@@ -18,8 +18,11 @@ through the public host-buffer path (pinned host memory -> H2D -> kernels -> row
 scan kernel against the measured HBM bandwidth; `cpu_baseline` (N = 1) and `--impl reference` time the UNMODIFIED
 reference (`python oracle/_ref/mCaller.py ... -t <cores>`, laid out by oracle/make_ref.sh) on a bounded sample of the
 same workload, and `parity_check` compares the GPU rows on that sample with the reference's and the oracle's.
+`--dump-outputs DIR` writes the rows and the histogram of the last timed step as .npy files: the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4] [--reads R] ...
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4] [--reads R]
+                    [--dump-outputs DIR] ...
 """
 import argparse
 import json
@@ -43,10 +46,17 @@ UNIT = "calls/s"
 BED_DEPTH, BED_THRESH = 15, 0.5           # make_bed.py -d 15 -t 0.5 (BASELINE configs[2])
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=10)
+    p.add_argument("--steps", type=positive_int, default=10, help="timed steps (of the main region and of the e2e leg)")
     p.add_argument("--warmup", type=int, default=3)
     p.add_argument("--impl", default="ours", choices=["ours", "reference"])
     p.add_argument("--config", type=int, default=0, choices=[0, 1, 2, 3, 4],
@@ -67,7 +77,12 @@ def parse_args():
     p.add_argument("--no-cpu", action="store_true")
     p.add_argument("--no-bind", action="store_true", help="do not bind the rank to a core set / NUMA node")
     p.add_argument("--budget-s", type=float, default=240.0, help="wall-clock budget of the reference arm's timed steps")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
+    a = p.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def resolve_config(args, world):
@@ -432,6 +447,55 @@ def parity_check(W, cfg, files, ref_diffs_path):
     return out
 
 
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_HEADER_BYTES = 128                   # per .npy file
+
+
+def dump_outputs(engine, cfg, out_dir):
+    """Writes what the last timed step computed, as a caller of the step receives it, to out_dir/<name>.npy:
+      rows_*  the step's `.diffs` rows (kind MC_CALL, in output order): byte offset of the read in the text, position,
+              strand (1 = '-'), the k + 1 features (empty columns are 0 with their bit set in rows_empty_mask), the
+              classifier's probability and label (1 = methylated);
+      hist_*  the per-site histogram (all-reduced over ranks): depth, methylated calls, first-seen global row index (-1:
+              no row), and with BED thresholds in the step the per-site selection flag.
+    float64, float32 where every value is a small integer.  Outputs larger than DUMP_BYTES keep a seeded sample of the rows
+    and of the site slots (the same entries on every run with the same arguments).  Returns a summary for the JSON line."""
+    from mcaller_b200 import _lib, engine as eng_mod
+    n_rows = int(engine.d_small[eng_mod.S_NROWS].item())
+    rows = engine._bufs["calls"][: n_rows * _lib.CALL_DTYPE.itemsize].cpu().numpy().view(_lib.CALL_DTYPE)
+    rows = rows[rows["kind"] == _lib.MC_CALL]
+    k1 = 7                                 # -n 6 current differences + the read quality
+    f64, f32 = np.float64, np.float32
+    row_cols = {"rows_read_offset": (rows["read_off"], f64), "rows_position": (rows["mpos"], f64), "rows_strand": (rows["rev"], f32),
+                "rows_features": (rows["feat"][:, :k1], f64), "rows_empty_mask": (rows["empty_mask"], f32),
+                "rows_probability": (rows["prob"], f64), "rows_label": (rows["label"], f32)}
+    ns = max(engine.ref.n_sites, 1)
+    first = engine.d_first.cpu().numpy()
+    first = np.where(first == 2 ** 63 - 1, -1, first)
+    site_cols = {"hist_depth": (engine.d_depth.cpu().numpy(), f32), "hist_methylated": (engine.d_meth.cpu().numpy(), f32),
+                 "hist_first_row": (first, f64)}
+    if cfg["bed"]:
+        site_cols["hist_bed_selected"] = (engine.d_bed_flags.cpu().numpy(), f32)
+
+    def width(cols):
+        return sum(np.dtype(dt).itemsize * int(np.prod(a.shape[1:])) for a, dt in cols.values())
+    total = len(rows) * width(row_cols) + ns * width(site_cols)
+    budget = DUMP_BYTES - DUMP_HEADER_BYTES * (len(row_cols) + len(site_cols))
+    scale = min(1.0, budget / total) if total else 1.0
+
+    def sample(n, seed):
+        keep = int(n * scale)
+        if keep >= n:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    row_idx, site_idx = sample(len(rows), 0), sample(ns, 1)
+    for cols, idx in ((row_cols, row_idx), (site_cols, site_idx)):
+        for name, (a, dt) in cols.items():
+            np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[idx], dtype=dt))
+    return {"dir": out_dir, "rows": len(rows), "rows_written": len(row_idx), "sites": ns, "sites_written": len(site_idx)}
+
+
 _REAL_STDOUT = None
 
 
@@ -601,6 +665,7 @@ def main():
     calls_per_step += int(n_odd[0])
     total_calls = calls_per_step * args.steps
     value = total_calls / (elapsed_ms / 1e3)
+    dumped = dump_outputs(engine, cfg, args.dump_outputs) if args.dump_outputs and rank == 0 else None
 
     # N > 1 runs configs[2] while the driver's N = 1 run is configs[1] (fewer calls per byte): so that the scaling of THIS
     # workload can be read off the line, rank 0 also times its own slice alone (no collectives, the other ranks wait)
@@ -693,7 +758,7 @@ def main():
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         e_calls = 0
-        e_steps = max(1, min(args.steps, 3))
+        e_steps = args.steps
         for _ in range(e_steps):
             e_calls += e2e_pass()
         torch.cuda.synchronize()
@@ -767,6 +832,8 @@ def main():
                            "binding": binding},
                 "clocks": clocks, "e2e": e2e, "gpu_launches": launches, "roofline": roofline, "cpu_baseline": cpu,
                 "parity_check": parity}
+        if dumped:
+            line["outputs_dumped"] = dumped
         emit_line(line)
     if use_dist:
         dist.destroy_process_group()

@@ -63,7 +63,7 @@ CASES = {
     "cg_c": dict(spec=_SPEC_G, motif="CG", model=R94, base="C", s=1),
     # the reference's alternative classifiers (-c RF / LR / NBC; pickles fitted by tools/make_alt_models.py, the reference
     # ships none): tree-walk, linear and naive-Bayes kernels pinned against the reference end to end
-    "rf_gatc": dict(spec=_SPEC3, motif="GATC", model="alt_RF_6_m6A.pkl", base="A", meth=True, s=1, classifier="RF"),
+    "rf_gatc": dict(spec=_SPEC3, motif="GATC", model="alt_RF_6_m6A.pkl.gz", base="A", meth=True, s=1, classifier="RF"),
     "lr_gatc": dict(spec=_SPEC3, motif="GATC", model="alt_LR_6_m6A.pkl", base="A", meth=True, classifier="LR"),
     "nbc_gatc": dict(spec=_SPEC3, motif="GATC", model="alt_NBC_6_m6A.pkl", base="A", meth=True, classifier="NBC"),
 }
@@ -165,6 +165,10 @@ def build_inputs(case, outdir, models_dir=None):
     models_dir = models_dir or os.path.join(GOLD, "models")
     paths = {"tsv": os.path.join(outdir, "syn.eventalign.tsv"), "fasta": os.path.join(outdir, "ref.fasta"),
              "fastq": os.path.join(outdir, "syn.fastq"), "model": os.path.join(models_dir, case["model"])}
+    if case["model"].endswith(".gz"):                      # large pickles are stored compressed; the runs read the plain file
+        paths["model"] = os.path.join(outdir, case["model"][:-3])
+        with gzip.open(os.path.join(models_dir, case["model"]), "rb") as src, open(paths["model"], "wb") as dst:
+            dst.write(src.read())
     if "fixture" in case:
         fx = os.path.join(GOLD, case["fixture"])
         tsv = gzip.open(os.path.join(fx, "masonread1.eventalign.tsv.gz"), "rb").read()
