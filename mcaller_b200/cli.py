@@ -11,14 +11,13 @@ concatenated, the per-site histograms are all-reduced over NCCL, and with `--bed
 straight from the combined histogram (`--bed_min_read_depth`, `--bed_mod_threshold`, `--bed_control`, `--bed_gff`,
 `--bed_ref` mirror make_bed.py's -d / -t / --control / --gff / --ref).
 """
-import math
 import os
 import sys
 from argparse import ArgumentParser
 
 
 def mcaller_main(argv=None):
-    from . import extract_contexts as ec, read_qual, refmark
+    from . import extract_contexts as ec, multigpu, read_qual, refmark
     p = ArgumentParser(description="Classify bases as methylated or unmethylated", prog="mCaller")
     g = p.add_mutually_exclusive_group(required=True)
     g.add_argument("-p", "--positions", type=str)
@@ -61,7 +60,6 @@ def mcaller_main(argv=None):
     assert os.path.isfile(a.fastq), "fastq file not found at " + a.fastq
     k = a.num_variables
     if a.gpus and a.gpus > 0:
-        from . import multigpu
         print("%d contigs" % len(refmark.read_fasta(a.reference)))
         print("%d GPUs" % a.gpus)
         multigpu.run(dict(tsv=a.tsv, reference=a.reference, fastq=a.fastq, modelfile=modelfile, k=k, skip=a.skip_thresh, qual=a.qual_thresh,
@@ -72,25 +70,15 @@ def mcaller_main(argv=None):
     read2qual = read_qual.extract_read_quality_device(a.fastq)        # FASTQ scanned on the GPU (same mapping as read_qual.py)
     print("%d contigs" % len(refmark.read_fasta(a.reference)))
     print("%d threads" % a.threads)
-    out = ".".join(a.tsv.split(".")[:-1]) + ".diffs." + str(k)
-    size = os.path.getsize(a.tsv)
-    n = max(1, a.threads)
-    chunk = int(math.ceil(size / float(n)))
-    tmps = []
-    for i in range(n):
-        start = chunk * i
-        tmp = out + ".tmp" + str(start)
+    ranges = multigpu.byte_ranges(os.path.getsize(a.tsv), max(1, a.threads))
+    for start, end in ranges:
+        tmp = multigpu.ec_tmp_name(a.tsv, k, start)
         if os.path.exists(tmp):
             os.remove(tmp)                       # the reference appends to stale files (quirk Q7); we start clean
         ec.extract_features(a.tsv, a.reference, read2qual, k, a.skip_thresh, a.qual_thresh, modelfile, a.classifier, start,
-                            endline=min(size, chunk * (i + 1)), train=False, base=base, motif=a.motif, positions_list=a.positions)
-        tmps.append(tmp)
+                            endline=end, train=False, base=base, motif=a.motif, positions_list=a.positions)
     print("Finished extracting signals")
-    with open(out, "wb") as dst:                 # ranges do not overlap: concatenation in offset order == -t 1 output
-        for tmp in tmps:
-            with open(tmp, "rb") as src:
-                dst.write(src.read())
-            os.remove(tmp)
+    multigpu.merge_outputs(a.tsv, k, len(ranges))
     return 0
 
 

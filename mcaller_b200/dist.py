@@ -48,8 +48,16 @@ def rank_row_base(rank):
 def close_and_reduce(engine, rank, group=None, fetch=True):
     """End of a rank's byte range in a multi-GPU run: close the window still open with the next rank's first kept line,
     then combine the histograms.  Returns the completed row (host array of one mc_call, kind MC_NONE when there was nothing
-    to close) when `fetch`."""
-    allk = gather_first_kept(engine.first_kept_contig_dev(), group)
+    to close) when `fetch`.  Under gloo (several ranks sharing one GPU) both exchanges are staged through host memory."""
+    host = dist.get_backend(group) == "gloo"
+    first_kept = engine.first_kept_contig_dev()
+    allk = gather_first_kept(first_kept.cpu() if host else first_kept, group).to(engine.device)
     row = engine.close_carry(next_contigs=allk, start=rank + 1, fetch=fetch)
-    allreduce_histogram(engine.d_counts, engine.d_first, group)
+    if host:
+        counts, first = engine.d_counts.cpu(), engine.d_first.cpu()
+        allreduce_histogram(counts, first, group)
+        engine.d_counts.copy_(counts)
+        engine.d_first.copy_(first)
+    else:
+        allreduce_histogram(engine.d_counts, engine.d_first, group)
     return row

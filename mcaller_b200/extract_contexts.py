@@ -58,6 +58,13 @@ def writefi(data, fi):
             outfi.write("\t".join(entry) + "\n")
 
 
+def diffs_name(tsv_input, k, start=None, train=False):
+    """`<tsv prefix>.diffs.<k>`, the merged output of a run; with `start`, the file the worker whose byte range starts there
+    appends to, `<tsv prefix>.diffs.<k>[.train].tmp<start>` (the reference's names)."""
+    stem = ".".join(tsv_input.split(".")[:-1]) + ".diffs." + str(k) + (".train" if train else "")
+    return stem if start is None else stem + ".tmp" + str(start)
+
+
 def base_models(base, twobase=False):
     """reference :99-106: two-letter context after the target -> model key."""
     if base == "A" and twobase:
@@ -177,157 +184,54 @@ def _fmt(x):
     return repr(float(x))
 
 
+def raise_row_error(err, mpos):
+    """The reference's failure for a window whose row carries MC_CE_* error flags."""
+    if err & 1:
+        raise ReferenceAbort("window at %d lies within k of a contig end (reference: IndexError / sys.exit at extract_contexts.py:195/:224)" % mpos)
+    if err & 2:
+        raise ReferenceAbort("base after target %d is not one of ACGTM (reference: KeyError -> sys.exit, :218-223)" % mpos)
+    if err & 4:
+        raise ValueError("unsupported numeric field in a line feeding the window at %d" % mpos)
+    if err & 16:
+        raise ReferenceAbort("n diffs off (multi-M spacing 0) at %d" % mpos)
+
+
 class _RowFormatter(object):
-    """Turns device rows into the reference's `.diffs.<k>` text rows (writer :216) and keeps the counters (:295-301).
+    """Training export: the closed call rows of a chunk as the reference's labelled `.diffs.<k>.train` rows (writer :216)
+    and the signal / context matrices train_model takes.  The carried window's read name and the counters are the
+    TextSink's (`sink`)."""
 
-    Row 0 of every chunk is the slot of the window carried over the chunk edge (mc_carry_rows): kind MC_NONE when empty,
-    else the completed row whose read name (read_off < 0) was kept here when the open row went by."""
-
-    def __init__(self, refindex, k, base, train, pos_label, have_model):
-        self.ref, self.k, self.base = refindex, k, base
-        self.train, self.pos_label, self.have_model = train, pos_label, have_model
-        self.mod_label = "m6A" if base == "A" else "m" + base
-        self.n_obs = 0
-        self.pos_set, self.multi, self.wskips, self.toomany = set(), set(), set(), set()
+    def __init__(self, refindex, k, pos_label, sink):
+        self.ref, self.k, self.pos_label, self.sink = refindex, k, pos_label, sink
         self.signals, self.contexts = {}, {}
-        self.pending = None        # (read name, segment key) of the window that is open across a chunk edge
-        self.seg_base = 0
-        self._native = None        # ctypes argument pack of mc_format_rows, built on first use
 
-    @staticmethod
-    def _check(err, mpos):
-        if err & 1:
-            raise ReferenceAbort("window at %d lies within k of a contig end (reference: IndexError / sys.exit at extract_contexts.py:195/:224)" % mpos)
-        if err & 2:
-            raise ReferenceAbort("base after target %d is not one of ACGTM (reference: KeyError -> sys.exit, :218-223)" % mpos)
-        if err & 4:
-            raise ValueError("unsupported numeric field in a line feeding the window at %d" % mpos)
-        if err & 16:
-            raise ReferenceAbort("n diffs off (multi-M spacing 0) at %d" % mpos)
-
-    def _row(self, c, read, segkey, chrom_idx):
+    def _row(self, c, read):
         k = self.k
         mpos = int(c["mpos"])
-        self._check(int(c["err"]), mpos)
+        raise_row_error(int(c["err"]), mpos)
         rev = bool(c["rev"])
         ctx = self.ref.context(int(c["win_contig"]), mpos, rev)
         em = int(c["empty_mask"])
         feat = c["feat"]
         feats = ["0" if (em >> j) & 1 else _fmt(feat[j]) for j in range(k)] + [_fmt(feat[k])]
-        chrom = self.ref.names[chrom_idx]
-        row = [chrom, read.decode(), str(mpos), ctx, ",".join(feats), strand(rev)]
-        if self.train:
-            label = self.pos_label[(chrom, mpos, strand(rev))]
-            row.append(label)
-            self.signals.setdefault("general", {}).setdefault(label, []).append([float(x) for x in feat[:k + 1]])
-            self.contexts.setdefault("general", {}).setdefault(label, []).append(ctx)
-        elif self.have_model:
-            p = float(c["prob"])
-            row.append(self.mod_label if p >= 0.5 else self.base)
-            row.append(str(np.round(np.float64(p), 2)))
-        self.n_obs += 1
-        self.pos_set.add(mpos)
-        if int(c["n_empty"]) > 0:
-            self.wskips.add((segkey << 32) | mpos)
-        return row
+        chrom = self.ref.names[int(c["chrom_contig"])]
+        label = self.pos_label[(chrom, mpos, strand(rev))]
+        self.signals.setdefault("general", {}).setdefault(label, []).append([float(x) for x in feat[:k + 1]])
+        self.contexts.setdefault("general", {}).setdefault(label, []).append(ctx)
+        return [chrom, read.decode(), str(mpos), ctx, ",".join(feats), strand(rev), label]
 
-    def _native_args(self):
+    def consume(self, calls, host_text_ptr, n_segments):
+        """Rows of one chunk (host structured array, slot 0 first; read names at host_text_ptr) -> list of row lists."""
         import ctypes as C
-        if self._native is None:
-            names = self.ref.names
-            n = len(names)
-            keep = [nm.encode() for nm in names] + list(self.ref.marked_bytes(0)) + list(self.ref.marked_bytes(1))
-            self._native = dict(keep=keep, names=(C.c_char_p * n)(*keep[:n]), fwd=(C.c_char_p * n)(*keep[n:2 * n]),
-                                rev=(C.c_char_p * n)(*keep[2 * n:]), lens=(C.c_int64 * n)(*[len(x) for x in keep[n:2 * n]]), n=n)
-        return self._native
-
-    def _segkeys(self, calls):
-        """Segment key of every row: chunk-local segment + the segments of earlier chunks; the carried row keeps the key it
-        had when it was opened."""
-        segkey = calls["seg"].astype(np.int64) + self.seg_base
-        carried = calls["read_off"] < 0
-        if carried.any():
-            segkey[carried] = self.pending[1] if self.pending is not None else -1
-        return segkey
-
-    def consume_bytes(self, calls, text, n_segments):
-        """Rows of one chunk (host structured array, slot 0 first) -> bytes of `.diffs` text rendered by the native writer
-        (mc_format_rows); counters are updated with vectorised numpy operations.  Inference mode only."""
-        import ctypes as C
-        from . import _lib
-        n = len(calls)
-        if n == 0:
-            self.seg_base += n_segments
-            return b""
-        kind = calls["kind"]
-        pend = calls["close_rec"] == _lib.PENDING
-        segkey = self._segkeys(calls)
-        pair = (segkey << 32) | calls["mpos"].astype(np.int64)
-        closed0 = (kind == _lib.MC_CALL) & ~pend
-        self.multi.update(np.unique(pair[kind == _lib.MC_MULTI_M]).tolist())
-        self.toomany.update(np.unique(pair[(kind == _lib.MC_TOO_MANY_SKIPS) & ~pend]).tolist())
-        self.wskips.update(np.unique(pair[closed0 & (calls["n_empty"] > 0)]).tolist())
-        self.pos_set.update(np.unique(calls["mpos"][closed0]).tolist())
-        self.n_obs += int(closed0.sum())
-        name, nlen = (self.pending[0], len(self.pending[0])) if self.pending is not None else (None, 0)
-        a = self._native_args()
-        L = _lib.lib()
-        cap = int(closed0.sum()) * (96 + 26 * (self.k + 1) + max(int(calls["read_len"].max()), nlen)) + 4096
-        out = C.create_string_buffer(cap)
-        if isinstance(text, np.ndarray):             # pinned host buffer of the streaming path: no copy
-            tbuf = C.c_void_p(text.ctypes.data)
-        else:
-            tbuf = (C.c_char * max(len(text), 1)).from_buffer_copy(text or b"\0") if not isinstance(text, (bytes, bytearray)) else text
-        calls_c = np.ascontiguousarray(calls)
-        r = L.mc_format_rows(calls_c.ctypes.data_as(C.c_void_p), n, tbuf, name, nlen, a["names"], a["fwd"], a["rev"], a["lens"], a["n"], self.k,
-                             self.base.encode(), self.mod_label.encode(), 1 if self.have_model else 0, 0, out, cap)
-        if r <= -100:
-            bad = calls[closed0 & (calls["err"] != 0)][0]
-            self._check(int(bad["err"]), int(bad["mpos"]))
-        if r < 0:
-            try:
-                _lib.check(int(r))
-            except _lib.McallerCudaError as e:
-                if "outside ACGTNM" in str(e):
-                    raise KeyError(str(e))               # the reference: KeyError in revcomp (:11-15)
-                raise
-        if kind[0] != _lib.MC_NONE and calls["read_off"][0] < 0:
-            self.pending = None                          # the carried window is written (or counted)
-        last = calls[n - 1]
-        if pend[n - 1] and kind[n - 1] != _lib.MC_MULTI_M and last["read_off"] >= 0:
-            ro = int(last["read_off"])
-            self.pending = (bytes(text[ro:ro + int(last["read_len"])]), int(segkey[n - 1]))
-        self.seg_base += n_segments
-        return out.raw[:r]
-
-    def consume(self, calls, text, n_segments):
-        """Rows of one chunk (host structured array, slot 0 first) -> list of row lists (Python path: training mode)."""
         from . import _lib
         out = []
         for c in calls:
-            kind = int(c["kind"])
-            if kind == _lib.MC_NONE:
+            if int(c["kind"]) != _lib.MC_CALL or int(c["close_rec"]) == _lib.PENDING:
                 continue
-            carried = int(c["read_off"]) < 0
-            if carried:
-                read, segkey = self.pending
-                self.pending = None
-            else:
-                segkey = self.seg_base + int(c["seg"])
-            if kind == _lib.MC_MULTI_M:
-                self.multi.add((segkey << 32) | int(c["mpos"]))
-                continue
-            if not carried:
-                ro = int(c["read_off"])
-                read = bytes(text[ro:ro + int(c["read_len"])])
-            if int(c["close_rec"]) == _lib.PENDING:
-                self.pending = (read, segkey)                # still open at the end of the chunk
-                continue
-            if kind == _lib.MC_TOO_MANY_SKIPS:
-                self.toomany.add((segkey << 32) | int(c["mpos"]))
-                continue
-            out.append(self._row(c, read, segkey, int(c["chrom_contig"])))
-        self.seg_base += n_segments
+            ro = int(c["read_off"])
+            read = self.sink.carry[0] if ro < 0 else C.string_at(host_text_ptr + ro, int(c["read_len"]))
+            out.append(self._row(c, read))
+        self.sink.advance(calls, host_text_ptr, n_segments)
         return out
 
 
@@ -348,14 +252,14 @@ def _select_device(startline, endline):
 
 
 class RangeRun(object):
-    """One worker's byte range of an eventalign file on one GPU: reference index, models, engine and row formatter, the
+    """One worker's byte range of an eventalign file on one GPU: reference index, models, engine and row writer, the
     streaming of the range into `<prefix>.diffs.<k>[.train].tmp<startline>` and the ways its last open window gets closed
     (probing the text after the range -- forked workers that cannot talk to each other -- or the next rank's first kept
     line in a multi-GPU run, mcaller_b200.multigpu)."""
 
     def __init__(self, tsv_input, fasta_input, read2qual, k, skip_thresh, qual_thresh, modelfile, startline, endline=None, train=False,
                  pos_label=None, base=None, motif=None, positions_list=None, histogram=False, row_base=0):
-        from . import engine as _engine, models as _models, read_qual as _rq
+        from . import engine as _engine, models as _models, read_qual as _rq, stream as _stream
         from .refindex import ReferenceIndex
         _engine.require_cuda()
         self.device_index = _select_device(startline, endline)
@@ -368,16 +272,13 @@ class RangeRun(object):
             print(str(e) + " - quitting thread now")
             raise ReferenceAbort(str(e))
         dm, two = None, False
-        stem = ".".join(tsv_input.split(".")[:-1]) + ".diffs." + str(k)
+        self.tsv_output = diffs_name(tsv_input, k, startline, train)
         if not train:
-            self.tsv_output = stem + ".tmp" + str(startline)
             model = _models.load_model_file(modelfile)
             e0, e1, two = _models.select_models(model, base)
             dm = _models.DeviceModels(e0, e1)
             if dm.n_in != k + 1:
                 raise ValueError("model expects %d inputs but -n %d gives %d" % (dm.n_in, k, k + 1))
-        else:
-            self.tsv_output = stem + ".train.tmp" + str(startline)
         # read2qual: the reference's dict, or a read_qual.DeviceQualityTable built on the GPU from the FASTQ
         qt = read2qual if isinstance(read2qual, _rq.DeviceQualityTable) else _rq.build_quality_table(read2qual)
         if isinstance(qt, _rq.DeviceQualityTable) and qt.table.device.index != self.device_index:
@@ -386,7 +287,8 @@ class RangeRun(object):
                                   histogram=histogram and dm is not None)
         if row_base:
             self.eng.reset_stream_state(row_base)
-        self.fmt = _RowFormatter(self.ref, k, base, train, pos_label, dm is not None)
+        self.sink = _stream.TextSink(self.ref, k, base, with_prob=dm is not None)
+        self.fmt = _RowFormatter(self.ref, k, pos_label, self.sink) if train else None
         self.fsize = os.path.getsize(tsv_input)
         if endline is None:
             endline = self.fsize
@@ -395,54 +297,32 @@ class RangeRun(object):
             self.hi = read_boundary_after(fh, min(endline, self.fsize), self.fsize)
         self.bytes_done = 0
 
-    def _write(self, rows):
-        if isinstance(rows, bytes):
-            with open(self.tsv_output, "ab") as outfi:          # append, like writefi (:83-86)
-                outfi.write(rows)
-        else:
-            writefi(rows, self.tsv_output)
+    def _render(self, h_calls, n_calls, host_text_ptr, n_segments=0):
+        """Rows of one chunk, or the completed carried row, appended to the tmp file (like writefi, :83-86)."""
+        from . import stream as _stream
+        if self.train:
+            writefi(self.fmt.consume(_stream.row_view(h_calls, n_calls), host_text_ptr, n_segments), self.tsv_output)
+            return
+        r = self.sink.render(h_calls, n_calls, host_text_ptr, n_segments)
+        with open(self.tsv_output, "ab") as outfi:
+            outfi.write(memoryview(self.sink.out)[:r])
 
     def stream(self):
-        """Rows of the reads whose first line lies in [lo, hi) -> the tmp file."""
-        eng, fmt = self.eng, self.fmt
+        """Rows of the reads whose first line lies in [lo, hi) -> the tmp file: reader thread -> pinned buffers -> H2D on a
+        side stream -> kernels -> rows back -> writer."""
+        from . import stream as _stream
         open(self.tsv_output, "a").close()
-        if not self.train:
-            # inference: pipelined path (reader thread -> pinned buffers -> H2D on a side stream -> kernels -> native writer)
-            from . import stream as _stream
-            # chunk size: the configured one (1 GiB) for long ranges -- fewest per-chunk costs: 25.7 GB/s from the page cache
-            # against 19.6 GB/s with 256 MiB chunks --, 1/32 of a shorter range: pinning three 1.25 GiB host buffers costs a
-            # fresh process 3.4 s, three of 320 MiB 1.1 s, and reading, copying and computing still overlap
-            chunk = min(CHUNK_BYTES, max(32 << 20, (self.hi - self.lo + 31) // 32))
-            fs = _stream.FileStreamer(eng, chunk, read_boundary_before, readers=READ_THREADS)
-            with open(self.tsv_output, "ab") as outfi:
-                for res, text, n in fs.chunks(self.tsv_input, self.lo, self.hi):
-                    _raise_on_counters(res)
-                    self._check_marking(text)
-                    outfi.write(fmt.consume_bytes(res.calls(), text, res.n_segments))
-                    self.bytes_done += n
-            return
-        with open(self.tsv_input, "rb") as fh:                  # training export: rows as Python lists (labels, matrices)
-            pos, carry = self.lo, b""
-            while pos < self.hi or carry:
-                want = min(CHUNK_BYTES, self.hi - pos)
-                fh.seek(pos)
-                data = carry + fh.read(want)
-                pos += want
-                if pos < self.hi:
-                    cut = read_boundary_before(data, len(data))
-                    if cut == 0:            # a single read larger than the chunk: keep reading
-                        carry = data
-                        continue
-                    carry, data = data[cut:], data[:cut]
-                else:
-                    carry = b""
-                if not data:
-                    continue
-                res = eng.run_chunk(eng.upload(data), len(data))
-                _raise_on_counters(res)
-                self._check_marking(data)
-                self._write(fmt.consume(res.calls(), data, res.n_segments))
-                self.bytes_done += len(data)
+        # chunk size: the configured one (1 GiB) for long ranges -- fewest per-chunk costs: 25.7 GB/s from the page cache
+        # against 19.6 GB/s with 256 MiB chunks --, 1/32 of a shorter range: pinning three 1.25 GiB host buffers costs a
+        # fresh process 3.4 s, three of 320 MiB 1.1 s, and reading, copying and computing still overlap
+        chunk = min(CHUNK_BYTES, max(32 << 20, (self.hi - self.lo + 31) // 32))
+        fs = _stream.FileStreamer(self.eng, chunk, read_boundary_before, readers=READ_THREADS)
+
+        def check(res, text):
+            _raise_on_counters(res)
+            self._check_marking(text)
+        fs.run(self.tsv_input, self.lo, self.hi, render=self._render, check=check)
+        self.bytes_done += fs.h2d_bytes
 
     def _check_marking(self, text):
         """The reference marks a contig when the TSV first names it and quits on a bad positions row then
@@ -463,12 +343,12 @@ class RangeRun(object):
         window comes back completed as slot 0 (mc_carry_rows); the pieces' own rows belong to the next worker and are
         ignored, as are its input problems.  At the end of the file nothing closes it (reference: dropped, SURVEY.md Q3)."""
         from . import _lib
-        eng, fmt = self.eng, self.fmt
-        if fmt.pending is None or self.hi >= self.fsize:
+        eng = self.eng
+        if self.sink.carry is None or self.hi >= self.fsize:
             return
         with open(self.tsv_input, "rb") as fh:
             ppos, size = self.hi, 4 << 20
-            while fmt.pending is not None and ppos < self.fsize:
+            while ppos < self.fsize:
                 fh.seek(ppos)
                 probe = fh.read(size)
                 at_eof = ppos + len(probe) >= self.fsize
@@ -488,16 +368,16 @@ class RangeRun(object):
         """The carried window, completed (by close_by_probe or Engine.close_carry), goes to the end of the tmp file."""
         from . import _lib
         if len(row) and row[0]["kind"] != _lib.MC_NONE:
-            self._write(self.fmt.consume(row, b"", 0) if self.train else self.fmt.consume_bytes(row, b"", 0))
+            self._render(row.view(np.uint8), 1, 0)
 
     def print_counters(self):
-        fmt = self.fmt
+        sink = self.sink
         print("thread finished processing...:")
-        print("%d observations" % fmt.n_obs)
-        print("%d positions" % len(fmt.pos_set))
-        print("%d regions with multiple methylated bases" % len(fmt.multi))
-        print("%d observations with skips included" % len(fmt.wskips))
-        print("%d observations with too many skips" % len(fmt.toomany))
+        print("%d observations" % sink.n_obs)
+        print("%d positions" % len(sink.pos_set))
+        print("%d regions with multiple methylated bases" % len(sink.multi))
+        print("%d observations with skips included" % len(sink.wskips))
+        print("%d observations with too many skips" % len(sink.toomany))
 
 
 def extract_features(tsv_input, fasta_input, read2qual, k, skip_thresh, qual_thresh, modelfile, classifier, startline, endline=None,

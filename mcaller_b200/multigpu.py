@@ -34,7 +34,7 @@ def run_rank(rank, world, port, a, backend=None):
     import numpy as np
     import torch
     import torch.distributed as dist
-    from . import _lib, dist as mdist, extract_contexts as ec, make_bed as mb, read_qual
+    from . import dist as mdist, extract_contexts as ec, make_bed as mb, read_qual
     n_dev = torch.cuda.device_count()
     dev_index = rank % max(n_dev, 1)
     torch.cuda.set_device(dev_index)
@@ -67,31 +67,17 @@ def run_rank(rank, world, port, a, backend=None):
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
         print("rank %d: %.2f GB of eventalign text -> %d rows in %.2f s (%.1f GB/s, %.0f calls/s) on cuda:%d"
-              % (rank, run.bytes_done / 1e9, run.fmt.n_obs, dt, run.bytes_done / 1e9 / max(dt, 1e-9), run.fmt.n_obs / max(dt, 1e-9), dev_index))
+              % (rank, run.bytes_done / 1e9, run.sink.n_obs, dt, run.bytes_done / 1e9 / max(dt, 1e-9), run.sink.n_obs / max(dt, 1e-9), dev_index))
         eng = run.eng
-        # (1) the window still open at the end of my range <- the first kept line of the next rank that has one
-        first_kept = eng.first_kept_contig_dev()
-        if backend == "nccl":
-            allk = mdist.gather_first_kept(first_kept)
-        else:                                         # gloo: stage through the host
-            allk = mdist.gather_first_kept(first_kept.cpu()).to(eng.device)
-        row = eng.close_carry(next_contigs=allk, start=rank + 1)
-        run.consume_closed(row)
-        # (2) the histograms
-        if backend == "nccl":
-            mdist.allreduce_histogram(eng.d_counts, eng.d_first)
-            depth, meth, first = eng.histogram_host() if rank == 0 else (None, None, None)
-        else:
-            c, f = eng.d_counts.cpu(), eng.d_first.cpu()
-            mdist.allreduce_histogram(c, f)
-            ns = c.numel() // 2
-            depth, meth, first = c[:ns].numpy().view(np.uint32), c[ns:].numpy().view(np.uint32), f.numpy().view(np.uint64)
+        # the window still open at the end of my range <- the first kept line of the next rank that has one; the histograms
+        run.consume_closed(mdist.close_and_reduce(eng, rank))
         odd = [None] * world
         dist.all_gather_object(odd, eng.odd_rows())
         run.print_counters()
         if rank == 0 and a.get("bed"):
             odd_rows = np.concatenate(odd) if any(len(o) for o in odd) else None
-            out = mb.output_name(".".join(a["tsv"].split(".")[:-1]) + ".diffs." + str(a["k"]), None, a["bed_control"], a["bed_gff"])
+            out = mb.output_name(ec.diffs_name(a["tsv"], a["k"]), None, a["bed_control"], a["bed_gff"])
+            depth, meth, first = eng.histogram_host()
             mb.aggregate_from_histogram(run.ref, depth, meth, first, out, a["bed_depth"], a["bed_thresh"], control=a["bed_control"],
                                         gff=a["bed_gff"], ref=a["bed_ref"], odd_rows=odd_rows)
         dist.barrier()
@@ -102,13 +88,16 @@ def run_rank(rank, world, port, a, backend=None):
 
 
 def ec_tmp_name(tsv, k, start):
-    return ".".join(tsv.split(".")[:-1]) + ".diffs." + str(k) + ".tmp" + str(start)
+    """The file the rank (or `-t N` worker) whose byte range starts at `start` writes its rows to."""
+    from .extract_contexts import diffs_name
+    return diffs_name(tsv, k, start)
 
 
 def merge_outputs(tsv, k, world):
     """Ranges do not overlap: concatenation in offset order == the -t 1 `.diffs.<k>` (no sort | uniq as in mCaller.py:103-107)."""
+    from .extract_contexts import diffs_name
     size = os.path.getsize(tsv)
-    out = ".".join(tsv.split(".")[:-1]) + ".diffs." + str(k)
+    out = diffs_name(tsv, k)
     with open(out, "wb") as dst:
         for start, _ in byte_ranges(size, world):
             tmp = ec_tmp_name(tsv, k, start)

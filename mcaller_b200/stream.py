@@ -1,9 +1,15 @@
-"""Streaming a host-resident eventalign buffer through the Engine: read-aligned chunks, double-buffered H2D copies on
-a side stream overlapped with the kernels, results copied back per chunk.  This is the path a file-based run takes
-(host memory -> PCIe -> HBM -> kernels -> rows back), and what bench.py times as `e2e`."""
+"""Streaming eventalign text through the Engine: read-aligned chunks, double-buffered H2D copies on a side stream
+overlapped with the kernels, the rows of every chunk copied back and rendered as `.diffs` text one chunk behind the GPU
+(host memory -> PCIe -> HBM -> kernels -> rows back -> text).  The chunks come from a pinned host buffer (HostStreamer,
+what bench.py times as `e2e`) or from a file (FileStreamer, the CLI and extract_features); both run the same pipeline and
+the same writer (TextSink)."""
+import ctypes as C
+import time
+
 import numpy as np
 import torch
 
+from . import _lib
 from ._lib import CALL_DTYPE, MC_TEXT_PAD
 
 
@@ -26,66 +32,102 @@ def plan_chunks(read_offsets, total_bytes, chunk_bytes):
     return cuts
 
 
+def row_view(h_calls, n_calls):
+    """The first n_calls rows of a pinned uint8 tensor or numpy uint8 array as a structured array (no copy)."""
+    raw = h_calls.numpy() if isinstance(h_calls, torch.Tensor) else h_calls
+    return raw[:n_calls * CALL_DTYPE.itemsize].view(CALL_DTYPE)
+
+
 class TextSink(object):
     """Renders the rows of a chunk as `.diffs.<k>` text with the native writer (mc_format_rows, host threads) straight from
-    the pinned row buffer and the host copy of the TSV (read names are cut from it).  Used by HostStreamer one chunk behind
-    the GPU, so the formatting overlaps the next chunk's copy and kernels.  A window still open at the end of a chunk comes
-    back completed as slot 0 of a later chunk (mc_carry_rows); its read name lies in the earlier chunk's text, so the sink
-    keeps those few bytes when it sees the open row."""
+    the pinned row buffer and the host copy of the TSV (read names are cut from it), and keeps the reference's five
+    counters (extract_contexts.py:295-301).  Row 0 of every chunk is the slot of the window carried over the chunk edge
+    (mc_carry_rows): kind MC_NONE when empty, else the completed row (read_off < 0) whose read name lies in an earlier
+    chunk's text, so the sink keeps those bytes, and the row's read-segment key, when it sees the open row."""
 
     def __init__(self, refindex, k, base="A", with_prob=True, keep=False, max_threads=0):
-        import ctypes as C
         names = refindex.names
         n = len(names)
         self._keep = [nm.encode() for nm in names] + list(refindex.marked_bytes(0)) + list(refindex.marked_bytes(1))
         self.names, self.fwd, self.rev = (C.c_char_p * n)(*self._keep[:n]), (C.c_char_p * n)(*self._keep[n:2 * n]), (C.c_char_p * n)(*self._keep[2 * n:])
         self.lens = (C.c_int64 * n)(*[len(x) for x in self._keep[n:2 * n]])
+        self.name_len = max([len(x) for x in self._keep[:n]] + [0])
         self.n, self.k, self.with_prob = n, int(k), 1 if with_prob else 0
         self.base, self.mod = base.encode(), (b"m6A" if base == "A" else b"m" + base.encode())
         self.max_threads = int(max_threads)
         self.out = None
         self.text_bytes = 0
         self.render_seconds = 0.0             # host time spent in the native writer
-        self.carry_name = None                # read name of the window currently open across a chunk edge
+        self.carry = None                     # (read name, segment key) of the window currently open across a chunk edge
+        self.seg_base = 0                     # read segments of the chunks so far: segment keys are unique over the range
+        self.n_obs = 0
+        self.pos_set, self.multi, self.wskips, self.toomany = set(), set(), set(), set()
         self.kept = [] if keep else None      # rendered text per chunk (tests)
 
-    def reset(self):
-        self.carry_name = None
-        self.text_bytes = 0
-        if self.kept is not None:
-            self.kept = []
-
-    def render(self, h_calls, n_calls, host_text_ptr, max_read_len=256):
+    def render(self, h_calls, n_calls, host_text_ptr, n_segments=0):
         """h_calls: pinned uint8 tensor (or numpy uint8 array) holding n_calls rows; host_text_ptr: address of the chunk's
-        first byte in host memory (0 when the rows carry no read_off into a text, e.g. the row of Engine.close_carry)."""
-        import ctypes as C
-        from . import _lib
-        if n_calls <= 0:
-            return 0
-        raw = h_calls.numpy() if hasattr(h_calls, "numpy") and not isinstance(h_calls, np.ndarray) else h_calls
-        rows = raw[:n_calls * CALL_DTYPE.itemsize].view(CALL_DTYPE)
-        name = self.carry_name
-        nlen = len(name) if name is not None else 0
-        cap = n_calls * (96 + 26 * (self.k + 1) + max(max_read_len, nlen)) + 4096
-        if self.out is None or len(self.out) < cap:
-            self.out = C.create_string_buffer(int(cap * 1.25))
-        import time as _time
-        t0 = _time.perf_counter()
-        r = _lib.lib().mc_format_rows(C.c_void_p(rows.ctypes.data), n_calls, C.c_void_p(host_text_ptr), name, nlen, self.names, self.fwd,
-                                      self.rev, self.lens, self.n, self.k, self.base, self.mod, self.with_prob, self.max_threads,
-                                      self.out, len(self.out))
-        self.render_seconds += _time.perf_counter() - t0
-        if r < 0:
-            _lib.check(int(r) if r > -100 else -1)
-        if rows[0]["kind"] != _lib.MC_NONE and rows[0]["read_off"] < 0:
-            self.carry_name = None            # the carried window has been written (or counted) with this chunk
-        last = rows[n_calls - 1]
-        if last["close_rec"] == _lib.PENDING and last["kind"] in (_lib.MC_CALL, _lib.MC_TOO_MANY_SKIPS) and last["read_off"] >= 0:
-            self.carry_name = C.string_at(host_text_ptr + int(last["read_off"]), int(last["read_len"]))
-        self.text_bytes += int(r)
-        if self.kept is not None:
-            self.kept.append(self.out.raw[:r])
-        return int(r)
+        first byte in host memory (0 when the rows carry no read_off into a text, e.g. the row of Engine.close_carry).
+        Returns the number of bytes rendered into self.out; row errors raise what the reference raises."""
+        rows = row_view(h_calls, n_calls)
+        r = 0
+        if n_calls > 0:
+            name = self.carry[0] if self.carry is not None else None
+            nlen = len(name) if name is not None else 0
+            # per row at most: contig and read name, 2k-1 context letters, k+1 floats of <= 24 characters, label,
+            # probability, position, strand and separators
+            cap = n_calls * (96 + 26 * (self.k + 1) + self.name_len + max(int(rows["read_len"].max()), nlen)) + 4096
+            if self.out is None or len(self.out) < cap:
+                self.out = C.create_string_buffer(int(cap * 1.25))
+            t0 = time.perf_counter()
+            r = int(_lib.lib().mc_format_rows(C.c_void_p(rows.ctypes.data), n_calls, C.c_void_p(host_text_ptr), name, nlen, self.names,
+                                              self.fwd, self.rev, self.lens, self.n, self.k, self.base, self.mod, self.with_prob,
+                                              self.max_threads, self.out, len(self.out)))
+            self.render_seconds += time.perf_counter() - t0
+            if r < 0:
+                self._raise(r, rows)
+            self.text_bytes += r
+            if self.kept is not None:
+                self.kept.append(self.out.raw[:r])
+        self.advance(rows, host_text_ptr, n_segments)
+        return r
+
+    @staticmethod
+    def _raise(r, rows):
+        from .extract_contexts import raise_row_error
+        if r <= -100:
+            bad = rows[(rows["kind"] == _lib.MC_CALL) & (rows["close_rec"] != _lib.PENDING) & (rows["err"] != 0)][0]
+            raise_row_error(int(bad["err"]), int(bad["mpos"]))
+        try:
+            _lib.check(r)
+        except _lib.McallerCudaError as e:
+            if "outside ACGTNM" in str(e):
+                raise KeyError(str(e))               # the reference: KeyError in revcomp (extract_contexts.py:11-15)
+            raise
+
+    def advance(self, rows, host_text_ptr, n_segments):
+        """Counts one chunk's rows (vectorised) and moves the carried window on: the one completed in slot 0 is done, a
+        call or too-many-skips window still open after the last row is kept with its read name.  render calls it; the
+        training export, which writes its own rows, calls it directly."""
+        n = len(rows)
+        if n:
+            kind = rows["kind"]
+            pend = rows["close_rec"] == _lib.PENDING
+            carried = rows["read_off"] < 0
+            segkey = rows["seg"].astype(np.int64) + self.seg_base
+            segkey[carried] = self.carry[1] if self.carry is not None else -1
+            pair = (segkey << 32) | rows["mpos"].astype(np.int64)
+            closed = (kind == _lib.MC_CALL) & ~pend
+            self.multi.update(np.unique(pair[kind == _lib.MC_MULTI_M]).tolist())
+            self.toomany.update(np.unique(pair[(kind == _lib.MC_TOO_MANY_SKIPS) & ~pend]).tolist())
+            self.wskips.update(np.unique(pair[closed & (rows["n_empty"] > 0)]).tolist())
+            self.pos_set.update(np.unique(rows["mpos"][closed]).tolist())
+            self.n_obs += int(closed.sum())
+            if kind[0] != _lib.MC_NONE and carried[0]:
+                self.carry = None             # the carried window has been written (or counted) with this chunk
+            last = rows[n - 1]
+            if pend[n - 1] and kind[n - 1] in (_lib.MC_CALL, _lib.MC_TOO_MANY_SKIPS) and not carried[n - 1]:
+                self.carry = (C.string_at(host_text_ptr + int(last["read_off"]), int(last["read_len"])), int(segkey[n - 1]))
+        self.seg_base += n_segments
 
 
 def last_boundary(arr, total, boundary_before, span=1 << 22):
@@ -109,24 +151,108 @@ def last_boundary(arr, total, boundary_before, span=1 << 22):
         span *= 4
 
 
-class FileStreamer(object):
-    """A byte range of an eventalign file -> read-aligned chunks through the Engine, pipelined: a reader thread fills a ring
-    of pinned host buffers with parallel preads (cutting at the last read boundary and carrying the incomplete read into
-    the next buffer), the H2D copy of chunk i+1 runs on a side stream while chunk i is in the kernels, and the caller
-    renders chunk i's rows while the next copy is in flight.  `boundary_before(bytes) -> offset` finds the last read
-    boundary of a buffer (extract_contexts.read_boundary_before)."""
+class _Pipeline(object):
+    """The device side of both sources: double-buffered H2D staging of the text on a side stream (chunk i+1 is copied
+    while chunk i is in the kernels), Engine.run_chunk, the pinned D2H of the rows and their rendering one chunk behind."""
 
-    def __init__(self, engine, chunk_bytes, boundary_before, slots=3, readers=4):
+    def __init__(self, engine):
         self.eng, self.dev = engine, engine.device
-        self.chunk_bytes = int(chunk_bytes)
-        self.boundary_before = boundary_before
-        self.n_slots, self.readers = int(slots), int(readers)
-        self.pin = [None] * self.n_slots          # pinned uint8 tensors, grown on demand
         self.dbuf = [None, None]
         self.copy_stream = torch.cuda.Stream(device=self.dev)
         self.ready = [torch.cuda.Event() for _ in range(2)]
         self.free = [torch.cuda.Event() for _ in range(2)]
+        self.h_calls = None                   # pinned rows: chunk i-1 is rendered before chunk i's rows are copied in
+        self.calls_done = torch.cuda.Event()
         self.h2d_bytes = 0
+        self.d2h_bytes = 0
+
+    def _enqueue_copy(self, dslot, src, n):
+        cap = self.eng.padded_capacity(n)
+        if self.dbuf[dslot] is None or self.dbuf[dslot].numel() < cap:
+            self.free[dslot].synchronize()
+            self.dbuf[dslot] = torch.empty(int(cap * 1.1) + 4096, dtype=torch.uint8, device=self.dev)
+        with torch.cuda.stream(self.copy_stream):
+            self.copy_stream.wait_event(self.free[dslot])
+            self.dbuf[dslot][:n].copy_(src[:n], non_blocking=True)
+            self.dbuf[dslot][n:n + MC_TEXT_PAD + 16].fill_(10)
+            self.ready[dslot].record(self.copy_stream)
+        self.h2d_bytes += n
+
+    def _stream(self, chunks, render=None, check=None, fetch_calls=True):
+        """chunks: iterator of (pinned uint8 tensor with the chunk's text at [0, n), n, release or None).  check(res, text)
+        runs as soon as chunk i's kernels are done, before any of its rows is rendered; render(h_calls, n_calls,
+        host_text_ptr, n_segments) gets chunk i's rows once chunk i+1 is in the kernels' queue.  Chunk i-1 is rendered and
+        released before chunk i+1 is taken: a source that cuts its chunks out of a ring of buffers (FileStreamer) needs that
+        slot back to hand chunk i+1 over.  Windows open at a chunk end are carried on the device (Engine.d_carry); the one
+        still open after the last chunk is left for the caller (Engine.close_carry: next rank / end of file)."""
+        eng = self.eng
+        fetch_calls = fetch_calls or render is not None
+        cur = torch.cuda.current_stream(self.dev)
+        for e in self.free:
+            e.record(cur)
+        tot = dict(calls=0, too_many_skips=0, multi=0, errors=0, methylated=0, records=0, lines=0, rows=0)
+        late = None                                   # (n_calls, text address, n_segments, release) of chunk i-1
+
+        def finish(n_c, ptr, n_seg, release):
+            if render is not None:
+                if n_c:
+                    self.calls_done.synchronize()
+                render(self.h_calls, n_c, ptr, n_seg)
+            if release is not None:
+                release()
+        chunks = iter(chunks)
+        nxt = next(chunks, None)
+        if nxt is not None:
+            self._enqueue_copy(0, nxt[0], nxt[1])
+        st, i = None, 0
+        while nxt is not None:
+            src, n, release = nxt
+            if late is not None:
+                finish(*late)
+            nxt = next(chunks, None)
+            if nxt is not None:
+                self._enqueue_copy((i + 1) & 1, nxt[0], nxt[1])
+            cur.wait_event(self.ready[i & 1])
+            res = eng.run_chunk(self.dbuf[i & 1], n)
+            if check is not None:
+                check(res, src.numpy()[:n])
+            st = res.stats
+            n_c = res.n_calls if fetch_calls else 0
+            if n_c:
+                nb = n_c * CALL_DTYPE.itemsize
+                if self.h_calls is None or self.h_calls.numel() < nb:
+                    self.h_calls = torch.empty(int(nb * 1.5) + 4096, dtype=torch.uint8, pin_memory=True)
+                self.h_calls[:nb].copy_(res.calls_dev[:nb], non_blocking=True)
+                self.calls_done.record(cur)
+                self.d2h_bytes += nb
+            late = (n_c, src.data_ptr(), res.n_segments, release)
+            self.free[i & 1].record(cur)
+            for kx in ("calls", "too_many_skips", "multi", "errors", "methylated"):
+                tot[kx] += st[kx]
+            tot["records"] += res.n_records
+            tot["lines"] += res.counters["lines"]
+            tot["rows"] += res.n_calls
+            i += 1
+        cur.synchronize()
+        if late is not None:
+            finish(*late)
+        # the window (call or too-many-skips event) still open after the last chunk: Engine.close_carry decides its fate
+        tot["open_at_end"] = (st["pending"] + st["pending_too_many_skips"]) if st is not None else 0
+        return tot
+
+
+class FileStreamer(_Pipeline):
+    """A byte range of an eventalign file -> read-aligned chunks through the pipeline: a reader thread fills a ring of
+    pinned host buffers with parallel preads, cutting at the last read boundary and carrying the incomplete read into the
+    next buffer.  A buffer goes back to the reader once its chunk's rows are rendered (read names are cut from its text).
+    `boundary_before(bytes) -> offset` finds the last read boundary of a buffer (extract_contexts.read_boundary_before)."""
+
+    def __init__(self, engine, chunk_bytes, boundary_before, slots=3, readers=4):
+        _Pipeline.__init__(self, engine)
+        self.chunk_bytes = int(chunk_bytes)
+        self.boundary_before = boundary_before
+        self.n_slots, self.readers = int(slots), int(readers)
+        self.pin = [None] * self.n_slots          # pinned uint8 tensors, grown on demand
 
     def _ensure_pin(self, slot, nbytes, keep=0):
         t = self.pin[slot]
@@ -136,9 +262,6 @@ class FileStreamer(object):
                 nt[:keep].copy_(t[:keep])
             self.pin[slot] = nt
         return self.pin[slot]
-
-    def _last_boundary(self, arr, total):
-        return last_boundary(arr, total, self.boundary_before)
 
     def _producer(self, path, lo, hi, q_free, q_ready):
         import os
@@ -168,7 +291,7 @@ class FileStreamer(object):
                         pos += want
                         total = carry + want
                         if pos < hi:
-                            cut = self._last_boundary(arr, total)
+                            cut = last_boundary(arr, total, self.boundary_before)
                             if cut == 0:                     # a single read larger than the chunk: keep reading into this slot
                                 carry = total
                                 continue
@@ -187,21 +310,8 @@ class FileStreamer(object):
         except BaseException as e:                          # surfaces in the consumer
             q_ready.put(e)
 
-    def _enqueue_copy(self, dslot, slot, n):
-        cap = self.eng.padded_capacity(n)
-        if self.dbuf[dslot] is None or self.dbuf[dslot].numel() < cap:
-            self.free[dslot].synchronize()
-            self.dbuf[dslot] = torch.empty(int(cap * 1.1) + 4096, dtype=torch.uint8, device=self.dev)
-        with torch.cuda.stream(self.copy_stream):
-            self.copy_stream.wait_event(self.free[dslot])
-            self.dbuf[dslot][:n].copy_(self.pin[slot][:n], non_blocking=True)
-            self.dbuf[dslot][n:n + MC_TEXT_PAD + 16].fill_(10)
-            self.ready[dslot].record(self.copy_stream)
-        self.h2d_bytes += n
-
-    def chunks(self, path, lo, hi):
-        """Yields (ChunkResult, host text of the chunk as a uint8 numpy view, nbytes) in file order.  The view and the
-        result's device buffers are valid until the next item is requested."""
+    def run(self, path, lo, hi, render=None, check=None):
+        """Streams the file's bytes [lo, hi) (read-aligned) through the pipeline; returns the totals of _Pipeline._stream."""
         import queue
         import threading
         q_free, q_ready = queue.Queue(), queue.Queue()
@@ -210,110 +320,31 @@ class FileStreamer(object):
         th = threading.Thread(target=self._producer, args=(path, lo, hi, q_free, q_ready), daemon=True)
         th.start()
 
-        def take():
-            item = q_ready.get()
-            if isinstance(item, BaseException):
-                raise item
-            return item
-        cur = torch.cuda.current_stream(self.dev)
-        for e in self.free:
-            e.record(cur)
-        item = take()
-        if item is not None:
-            self._enqueue_copy(0, item[0], item[1])
-        i = 0
-        while item is not None:
-            nxt = take()
-            if nxt is not None:
-                self._enqueue_copy((i + 1) & 1, nxt[0], nxt[1])
-            slot, n = item
-            cur.wait_event(self.ready[i & 1])
-            res = self.eng.run_chunk(self.dbuf[i & 1], n)
-            yield res, self.pin[slot].numpy()[:n], n
-            self.free[i & 1].record(cur)
-            q_free.put(slot)
-            item = nxt
-            i += 1
+        def chunks():
+            while True:
+                item = q_ready.get()
+                if isinstance(item, BaseException):
+                    raise item
+                if item is None:
+                    return
+                slot, n = item
+                yield self.pin[slot], n, lambda s=slot: q_free.put(s)
+        tot = self._stream(chunks(), render=render, check=check)
         th.join()
+        return tot
 
 
-class HostStreamer(object):
+class HostStreamer(_Pipeline):
+    """Chunks are slices of a pinned host buffer at plan_chunks cuts (bench.py's e2e leg)."""
+
     def __init__(self, engine, chunk_bytes=1 << 30):
-        self.eng = engine
-        self.dev = engine.device
+        _Pipeline.__init__(self, engine)
         self.chunk_bytes = int(chunk_bytes)
-        cap = engine.padded_capacity(self.chunk_bytes)
-        self.dbuf = [torch.empty(cap, dtype=torch.uint8, device=self.dev) for _ in range(2)]
-        self.copy_stream = torch.cuda.Stream(device=self.dev)
-        self.ready = [torch.cuda.Event() for _ in range(2)]
-        self.free = [torch.cuda.Event() for _ in range(2)]
-        self.h_calls = [None, None]           # pinned row buffers, alternating so one can be rendered while the other fills
-        self.calls_done = [torch.cuda.Event() for _ in range(2)]
-        self.h2d_bytes = 0
-        self.d2h_bytes = 0
-
-    def _enqueue_copy(self, slot, host_buf, a, b):
-        n = b - a
-        if n > self.chunk_bytes:
-            raise ValueError("chunk of %d bytes exceeds the staging buffers (%d)" % (n, self.chunk_bytes))
-        with torch.cuda.stream(self.copy_stream):
-            self.copy_stream.wait_event(self.free[slot])
-            self.dbuf[slot][:n].copy_(host_buf[a:b], non_blocking=True)
-            self.dbuf[slot][n:n + MC_TEXT_PAD + 16].fill_(10)
-            self.ready[slot].record(self.copy_stream)
-        self.h2d_bytes += n
 
     def run(self, host_buf, cuts, fetch_calls=True, sink=None):
         """host_buf: pinned uint8 CPU tensor; cuts: chunk end offsets from plan_chunks.  Returns dict of totals; rows of
         every chunk are copied to pinned host memory when fetch_calls (the D2H leg of the end-to-end path) and, with a
-        TextSink, rendered as `.diffs` text one chunk behind the GPU.  Windows open at a chunk end are carried on the device
-        (Engine.d_carry) and appear, completed, as slot 0 of the next chunk with a kept line; the one still open after the
-        last chunk is left in the carry for the caller (Engine.close_carry: next rank / end of file)."""
-        eng = self.eng
-        fetch_calls = fetch_calls or sink is not None
-        late = None                                   # (slot, n_calls, chunk start) of the chunk whose rows are not rendered yet
-
-        def render(item):
-            slot_c, n_c, start = item
-            self.calls_done[slot_c].synchronize()
-            sink.render(self.h_calls[slot_c], n_c, host_buf.data_ptr() + start)
-        cur = torch.cuda.current_stream(self.dev)
-        for e in self.free:
-            e.record(cur)
-        tot = dict(calls=0, too_many_skips=0, multi=0, errors=0, methylated=0, records=0, lines=0, rows=0)
+        TextSink, rendered as `.diffs` text."""
         bounds = [0] + list(cuts)
-        if len(bounds) > 1:
-            self._enqueue_copy(0, host_buf, bounds[0], bounds[1])
-        st = None
-        for i in range(len(bounds) - 1):
-            slot = i & 1
-            if i + 2 < len(bounds):
-                self._enqueue_copy((i + 1) & 1, host_buf, bounds[i + 1], bounds[i + 2])
-            cur.wait_event(self.ready[slot])
-            n = bounds[i + 1] - bounds[i]
-            res = eng.run_chunk(self.dbuf[slot], n)
-            st = res.stats
-            if fetch_calls and res.n_calls:
-                nb = res.n_calls * CALL_DTYPE.itemsize
-                sc = i & 1
-                if self.h_calls[sc] is None or self.h_calls[sc].numel() < nb:
-                    self.h_calls[sc] = torch.empty(int(nb * 1.5) + 4096, dtype=torch.uint8, pin_memory=True)
-                self.h_calls[sc][:nb].copy_(res.calls_dev[:nb], non_blocking=True)
-                self.calls_done[sc].record(cur)
-                self.d2h_bytes += nb
-                if sink is not None:
-                    if late is not None:
-                        render(late)                  # the previous chunk's rows, while this chunk's copy-back is in flight
-                    late = (sc, res.n_calls, bounds[i])
-            self.free[slot].record(cur)
-            for kx in ("calls", "too_many_skips", "multi", "errors", "methylated"):
-                tot[kx] += st[kx]
-            tot["records"] += res.n_records
-            tot["lines"] += res.counters["lines"]
-            tot["rows"] += res.n_calls
-        cur.synchronize()
-        if sink is not None and late is not None:
-            render(late)
-        # the window (call or too-many-skips event) still open after the last chunk: Engine.close_carry decides its fate
-        tot["open_at_end"] = (st["pending"] + st["pending_too_many_skips"]) if st is not None else 0
-        return tot
+        return self._stream(((host_buf[a:b], b - a, None) for a, b in zip(bounds, bounds[1:])),
+                            render=sink.render if sink is not None else None, fetch_calls=fetch_calls)

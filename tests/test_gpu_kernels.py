@@ -613,12 +613,14 @@ def test_window_units_in_other_site_regimes(mode, tmp_path, cuda_lib, oracle):
     assert st["too_many_skips"] == want["counters"]["too_many_skips"] and st["multi"] == want["counters"]["multi"] and st["errors"] == 0
 
 
-def test_streamed_text_rows_match_oracle(cuda_lib, oracle):
+def test_streamed_text_rows_match_oracle(tmp_path, cuda_lib, oracle):
     """HostStreamer + TextSink (pinned host TSV -> H2D -> kernels -> rows D2H -> native multi-threaded writer): with one chunk
     the text is the oracle's `.diffs` rows byte for byte, and so it is with several chunks: a window open at a chunk edge is
-    carried on the device and written, completed, with the first rows of the next chunk."""
+    carried on the device and written, completed, with the first rows of the next chunk.  The same holds for FileStreamer
+    reading the TSV from disk in small chunks through its ring of three pinned buffers (each goes back to the reader only
+    after its chunk's rows are rendered)."""
     import torch
-    from mcaller_b200 import engine, models, read_qual, stream, synth
+    from mcaller_b200 import engine, extract_contexts as ec, models, read_qual, stream, synth
     from mcaller_b200.refindex import ReferenceIndex
     spec = synth.SynthSpec(seed=93, contigs=[("ecoli", 60000)], n_reads=400, len_min=400, len_max=1500)
     tsv, fasta, fastq, quals = synth.generate(spec)
@@ -650,6 +652,15 @@ def test_streamed_text_rows_match_oracle(cuda_lib, oracle):
         got = b"".join(sink.kept)
         assert len(cuts) == 1 or len(cuts) >= 4
         assert got == want_text
+    path = tmp_path / "syn.eventalign.tsv"
+    path.write_bytes(tsv)
+    fs = stream.FileStreamer(eng, len(tsv) // 40, ec.read_boundary_before, slots=3)
+    sink = stream.TextSink(ref, 6, "A", keep=True)
+    eng.reset_histogram()
+    tot = fs.run(str(path), 0, len(tsv), render=sink.render)
+    assert len(sink.kept) >= 30 and fs.h2d_bytes == len(tsv)
+    assert b"".join(sink.kept) == want_text
+    assert sink.n_obs == tot["calls"] == len(want["rows"])
 
 
 def test_fastq_quality_on_device_matches_host(tmp_path, cuda_lib):
