@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MC_ABI_VERSION 2
+#define MC_ABI_VERSION 3
 
 /* text chunks: one warp tokenises MC_TILE_BYTES of TSV; the caller must keep MC_TEXT_PAD readable bytes,
  * all '\n', after the last text byte (so a final line without newline and tile look-ahead are safe). */
@@ -361,13 +361,11 @@ typedef struct mc_locus_entry {
     uint32_t depth;
     uint32_t meth;
 } mc_locus_entry;
-int mc_diffs_aggregate(const uint8_t *d_text, int64_t nbytes, mc_locus_entry *d_table, int64_t table_size,
-                       uint64_t *d_counters, void *stream);
 
 /*
  * make_bed variants that need per-read lists (make_bed.py -p and --vo; SURVEY.md section 8f rank 3).
  *
- * mc_diffs_aggregate_ex: mc_diffs_aggregate with the `-p` filter of make_bed.py:73-74/:84 and a base offset, so a file can be
+ * mc_diffs_aggregate_ex: the aggregation above with the `-p` filter of make_bed.py:73-74/:84 and a base offset, so a file can be
  *   streamed in line-aligned pieces into one table (first_off = base_off + offset inside the piece) -- d_posset (may be NULL) is an
  *   open-addressing set (power-of-two entries, 0 = empty) of FNV-1a hashes of "chrom\tpos\tstrand" built by the host from
  *   the positions file (entries whose end column is not start + 1 can never match and are left out).

@@ -17,7 +17,7 @@ MC_MAXK = 8
 MC_C_COUNT = 16
 COUNTER_NAMES = ["lines", "kept", "records", "short", "unknown_contig", "nnn", "badpos", "longline", "overflow", "run_cursor", "quiet_chunks"]
 
-MC_ABI_VERSION = 2
+MC_ABI_VERSION = 3
 MC_CALL, MC_TOO_MANY_SKIPS, MC_MULTI_M, MC_NONE = 0, 1, 2, 3
 MC_CE_CONTEXT, MC_CE_MODELKEY, MC_CE_BADNUM, MC_CE_COLUMN, MC_CE_SPACING = 1, 2, 4, 8, 16
 MC_MLP, MC_LR, MC_GNB, MC_RF = 0, 1, 2, 3
@@ -132,7 +132,6 @@ _PROTOS = {
     "mc_synth_genome": (C.c_int, [C.POINTER(SynthSpec), C.c_void_p, C.c_int64, C.c_void_p]),
     "mc_synth_sizes": (C.c_int, [C.POINTER(SynthSpec), C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
     "mc_synth_write": (C.c_int, [C.POINTER(SynthSpec), C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "mc_diffs_aggregate": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "mc_diffs_aggregate_ex": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "mc_diffs_rehash": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "mc_diffs_rows": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,

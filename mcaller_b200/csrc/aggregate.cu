@@ -347,11 +347,6 @@ extern "C" int mc_diffs_aggregate_ex(const uint8_t *d_text, int64_t nbytes, int6
     return MC_OK;
 }
 
-extern "C" int mc_diffs_aggregate(const uint8_t *d_text, int64_t nbytes, mc_locus_entry *d_table, int64_t table_size,
-                                  uint64_t *d_counters, void *stream) {
-    return mc_diffs_aggregate_ex(d_text, nbytes, 0, nullptr, 0, d_table, table_size, d_counters, stream);
-}
-
 extern "C" int mc_diffs_rehash(const mc_locus_entry *d_old, int64_t old_size, mc_locus_entry *d_table, int64_t table_size,
                                uint64_t *d_counters, void *stream) {
     MC_REQUIRE(d_old && d_table && d_counters, "null pointer");

@@ -65,17 +65,40 @@ __device__ __forceinline__ int mc_block_exscan(int v, int *s_warp /* [THREADS/32
     return res;
 }
 
-// generic device exclusive scan (uint32 in -> uint32 out), see scan_util.cu
-int mc_exscan_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n, uint64_t *d_total /* may be null */, void *d_ws,
-                  cudaStream_t st);
-int mc_exscan_u32_dev(const uint32_t *d_in, uint32_t *d_out, int64_t n_cap, const uint64_t *d_n, uint64_t *d_total, void *d_ws,
-                      cudaStream_t st);
+// device exclusive scan (uint32 in -> uint32 out, records.cu) of n_cap items, or of the first *d_n of them when the count
+// lives on the device (items beyond it count as zero); d_total (may be null) receives the sum
+int mc_exscan_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n_cap, const uint64_t *d_n /* may be null */,
+                  uint64_t *d_total /* may be null */, void *d_ws, cudaStream_t st);
 int64_t mc_exscan_ws_bytes(int64_t n);
 
 // item count kept on the device (stage outputs), clamped to the capacity the launch was sized for
 __device__ __forceinline__ int64_t mc_dev_count(const unsigned long long *d_n, int64_t cap) {
     const unsigned long long v = *d_n;
     return v < (unsigned long long)cap ? (int64_t)v : cap;
+}
+
+// byte offset of a record's line in the text
+__device__ __forceinline__ int64_t mc_rec_line(const mc_record &r) { return ((int64_t)r.line_hi << 32) | (int64_t)r.line_lo; }
+
+// Read-quality key of a read name: name.split(':')[0].split('_')[0] (read_qual.py:11-12 / extract_contexts.py:166), the
+// bytes at p up to whitespace, ':' or '_' (at most max_len of them), hashed by FNV-1a with two bases.  The fastq ingest
+// (k_fq_insert) builds its table and stage 4 (k_seg_quality) probes it with this one function; the host twin is
+// read_qual.fnv_pair.
+struct mc_read_key {
+    unsigned long long hash;   // never 0 (0 marks an empty table slot)
+    uint32_t check;            // high word of the second hash
+    uint32_t len;
+};
+__device__ __forceinline__ mc_read_key mc_read_key_of(const uint8_t *p, int64_t max_len) {
+    unsigned long long h = 14695981039346656037ull, h2 = 0x84222325cbf29ce4ull;
+    int64_t len = 0;
+    for (; len < max_len; ++len) {
+        const unsigned c = __ldg(p + len);
+        if (c <= 0x20u || c == ':' || c == '_') break;
+        h = (h ^ c) * 1099511628211ull;
+        h2 = (h2 ^ c) * 1099511628211ull;
+    }
+    return {h == 0ull ? 1ull : h, (uint32_t)(h2 >> 32), (uint32_t)len};
 }
 
 // numpy's pairwise summation (np.add.reduce over a contiguous float64 vector) of f(x_i), i in [i0, i0 + n):

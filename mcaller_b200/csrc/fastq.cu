@@ -82,17 +82,8 @@ __global__ void __launch_bounds__(256) k_fq_insert(const uint8_t *__restrict__ t
     if (lane != 0) return;
     if (__ldg(text + h0) != '@') { atomicAdd(&d_stats[1], 1ull); return; }             // not a FASTQ header
     // id = first whitespace-delimited token after '@'; key = id up to the first ':' or '_'
-    unsigned long long h = 14695981039346656037ull, h2 = 0x84222325cbf29ce4ull;
-    uint32_t len = 0;
-    for (unsigned long long p = h0 + 1; p < h1; ++p) {
-        const unsigned c = __ldg(text + p);
-        if (c <= 0x20u || c == ':' || c == '_') break;
-        h = (h ^ c) * 1099511628211ull;
-        h2 = (h2 ^ c) * 1099511628211ull;
-        ++len;
-    }
-    if (h == 0ull) h = 1ull;
-    const uint32_t check = (uint32_t)(h2 >> 32);
+    const mc_read_key key = mc_read_key_of(text + h0 + 1, (int64_t)(h1 - h0) - 1);
+    const unsigned long long h = key.hash;
     const double mean = qlen > 0 ? __ddiv_rn((double)(sum - 33ull * (unsigned long long)qlen), (double)qlen)
                                  : __longlong_as_double(0x7ff8000000000000ll);          // np.mean([]) is nan
     rec_mean[rec] = mean;
@@ -103,8 +94,8 @@ __global__ void __launch_bounds__(256) k_fq_insert(const uint8_t *__restrict__ t
         if (cur == 0ull) {
             cur = atomicCAS(hp, 0ull, h);
             if (cur == 0ull) {                       // claimed: publish the rest of the key
-                table[slot].check = check;
-                table[slot].len = len;
+                table[slot].check = key.check;
+                table[slot].len = key.len;
                 cur = h;
             }
         }
@@ -141,7 +132,7 @@ extern "C" int mc_fastq_index(const uint8_t *d_text, int64_t nbytes, uint32_t *d
     if (nt == 0) { MC_CUDA_CHECK(cudaMemsetAsync(d_n_newlines, 0, 8, st)); return MC_OK; }
     k_fq_count<<<(unsigned)nt, FQ_THREADS, 0, st>>>(d_text, nbytes, d_tile_cnt);
     MC_LAUNCH_CHECK();
-    int rc = mc_exscan_u32(d_tile_cnt, d_tile_off, nt, d_n_newlines, d_ws, st);
+    int rc = mc_exscan_u32(d_tile_cnt, d_tile_off, nt, nullptr, d_n_newlines, d_ws, st);
     if (rc) return rc;
     k_fq_lines<<<(unsigned)nt, FQ_THREADS, 0, st>>>(d_text, nbytes, d_tile_off, reinterpret_cast<unsigned long long *>(d_line_start),
                                                     (unsigned long long)line_cap);

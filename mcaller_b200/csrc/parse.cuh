@@ -113,6 +113,30 @@ __device__ __forceinline__ void parse_values(const B &t, int f2, int f5, int f6,
     if (tokens_equal(t, f2, f9)) flags |= MC_RF_EQ;
 }
 
+// ---- byte and bit helpers in registers -------------------------------------------------------------------------------------
+// 0x80 per byte of w that is > 0x20 (not whitespace)
+__device__ __forceinline__ uint32_t gt20_msb(uint32_t w) { return (((w & 0x7f7f7f7fu) + 0x5f5f5f5fu) | w) & 0x80808080u; }
+// 4 msb-form words (0x80 per flagged byte) -> 16 flag bits in byte order.  IDP.4A sums 0x80 * weight per byte: two words
+// fill bits 7..14 of one accumulator.
+__device__ __forceinline__ uint32_t pack16(uint32_t m0, uint32_t m1, uint32_t m2, uint32_t m3) {
+    const uint32_t lo = 0x08040201u, hi = 0x80402010u;
+    const uint32_t a = __dp4a(m1, hi, __dp4a(m0, lo, 0u)), b = __dp4a(m3, hi, __dp4a(m2, lo, 0u));
+    return (a >> 7) | (b << 1);
+}
+// position of the j-th (0-based) set bit of m, j < popc(m)
+__device__ __forceinline__ int nth_bit(uint32_t m, int j) {
+#pragma unroll
+    for (int t = 0; t < 6; ++t)
+        if (j > t) m &= m - 1u;
+    for (int t = 6; t < j; ++t) m &= m - 1u;                     // words with more than 7 set bits: rare
+    return __ffs(m) - 1;
+}
+// 4 digit values, most significant in byte 0 -> 0..9999
+__device__ __forceinline__ uint32_t conv4(uint32_t h) {
+    const uint32_t t = ((h * 2561u) >> 8) & 0x00ff00ffu;
+    return (t * 6553601u) >> 16;
+}
+
 // ---- 8-byte register fast paths for the values of a record (any other shape falls back to the byte loops of parse.cuh) ----
 // 0x80 per byte of v that is not an ASCII digit
 __device__ __forceinline__ unsigned long long nondigit8(unsigned long long v) {
@@ -122,12 +146,7 @@ __device__ __forceinline__ unsigned long long nondigit8(unsigned long long v) {
 // n (1..7) digit bytes at the low end of v -> value
 __device__ __forceinline__ uint32_t digits_value(unsigned long long v, int n) {
     const unsigned long long x = (v ^ 0x3030303030303030ull) << (64 - 8 * n);      // right-aligned digit values, zeros below
-    const uint32_t L = (uint32_t)x, H = (uint32_t)(x >> 32);
-    auto conv4 = [](uint32_t h) {                                 // 4 digit values, most significant in byte 0 -> 0..9999
-        const uint32_t t = ((h * 2561u) >> 8) & 0x00ff00ffu;
-        return (t * 6553601u) >> 16;
-    };
-    return conv4(L) * 10000u + conv4(H);
+    return conv4((uint32_t)x) * 10000u + conv4((uint32_t)(x >> 32));
 }
 // "<1..7 digits><ws>" -> value; false for any other shape
 __device__ __forceinline__ bool fast_uint8(unsigned long long v, int &out) {
@@ -166,13 +185,7 @@ __device__ __forceinline__ int fast_tokens_equal8(unsigned long long a, unsigned
     return (((a ^ b) & ((1ull << (8 * la)) - 1ull)) == 0ull) ? 1 : 0;
 }
 
-// ---- finishing a raw record from the text in global memory (shared by stage 1's batched flush and stage 2) ------------------
-__device__ __forceinline__ uint32_t fin_gt20(uint32_t w) { return (((w & 0x7f7f7f7fu) + 0x5f5f5f5fu) | w) & 0x80808080u; }
-__device__ __forceinline__ uint32_t fin_pack16(uint32_t m0, uint32_t m1, uint32_t m2, uint32_t m3) {
-    const uint32_t lo = 0x08040201u, hi = 0x80402010u;
-    const uint32_t a = __dp4a(m1, hi, __dp4a(m0, lo, 0u)), b = __dp4a(m3, hi, __dp4a(m2, lo, 0u));
-    return (a >> 7) | (b << 1);
-}
+// ---- finishing a raw record of stage 1 from the text in global memory (stage 2) ----------------------------------------------
 // 8 bytes at any alignment from two aligned 8-byte loads
 __device__ __forceinline__ unsigned long long load8_unaligned(const uint8_t *p) {
     const uintptr_t a = reinterpret_cast<uintptr_t>(p);
@@ -205,13 +218,30 @@ __device__ __forceinline__ bool bytes_differ(const uint8_t *pa, const uint8_t *p
     return diff != 0ull;
 }
 
+// Event index (column 6), np.round(event_mean - model_mean, 4) (7, 11) and the k-mer equality flag (3 vs 10) of the line
+// at lp, of which `room` bytes are readable; f2..f10 are the line offsets of those columns.  The usual shapes ("1234",
+// "87.41", 6-mers) are decoded from 8-byte register loads, anything else by the byte loops of parse_values -- both give
+// the same float64.
+__device__ __forceinline__ void mc_finish_values(const uint8_t *lp, int64_t room, int f2, int f5, int f6, int f9, int f10, int &ev_idx,
+                                                 double &diff, uint32_t &fl) {
+    uint32_t m_ev = 0u, m_md = 0u;
+    int n_ev = 0, n_md = 0;
+    const int teq = fast_tokens_equal8(load8_unaligned(lp + f2), load8_unaligned(lp + f9));
+    if (f10 + 16 < room && teq >= 0 && fast_uint8(load8_unaligned(lp + f5), ev_idx) &&
+        fast_decimal8(load8_unaligned(lp + f6), m_ev, n_ev) && fast_decimal8(load8_unaligned(lp + f10), m_md, n_md)) {
+        const double ev = __ddiv_rn((double)m_ev, c_pow10[n_ev]), md = __ddiv_rn((double)m_md, c_pow10[n_md]);
+        diff = __ddiv_rn(rint(__dmul_rn(__dsub_rn(ev, md), 1e4)), 1e4);
+        if (teq) fl |= MC_RF_EQ;
+    } else {
+        parse_values(GlobalBytes{lp, room}, f2, f5, f6, f9, f10, ev_idx, diff, fl);
+    }
+}
+
 // Walks the columns of the record's line in the text (16-byte SWAR steps over the non-whitespace map; columns split on
 // runs of bytes <= 0x20 like str.split(), extract_contexts.py:150) and parses what the window builder needs: read-name span
-// (column 4), event index (6), np.round(event_mean - model_mean, 4) (7, 11) and the k-mer equality flag (3 vs 10).  The usual
-// shapes ("1234", "87.41", 6-mers) are decoded from 8-byte register loads, anything else by the byte loops above -- both
-// give the same float64.  Clears MC_RF_RAW.
+// (column 4) and the values of mc_finish_values.  Clears MC_RF_RAW.
 __device__ __forceinline__ void mc_finish_record(const uint8_t *__restrict__ text, int64_t limit, mc_record &r) {
-    const int64_t line = ((int64_t)r.line_hi << 32) | (int64_t)r.line_lo;
+    const int64_t line = mc_rec_line(r);
     // 16-byte steps from the aligned address at or below the line start; the '\n' padding after the text makes every
     // line end inside readable memory
     const int64_t a0 = line & ~15ll;
@@ -224,7 +254,7 @@ __device__ __forceinline__ void mc_finish_record(const uint8_t *__restrict__ tex
         const int64_t g = a0 + 16ll * step;
         if (g >= limit) break;
         const uint4 v = __ldg(reinterpret_cast<const uint4 *>(text + g));
-        uint32_t nonws = fin_pack16(fin_gt20(v.x), fin_gt20(v.y), fin_gt20(v.z), fin_gt20(v.w));
+        uint32_t nonws = pack16(gt20_msb(v.x), gt20_msb(v.y), gt20_msb(v.z), gt20_msb(v.w));
         if (step == 0) nonws &= 0xFFFFu << skip;                 // ignore the bytes before the line start
         // no newline test: a recorded line is a kept line, its first 12 columns start before its end (stage 1 checked), so
         // the walk stops at the 11th column; MAX_STEPS bounds it for records that did not come from stage 1
@@ -261,22 +291,7 @@ __device__ __forceinline__ void mc_finish_record(const uint8_t *__restrict__ tex
     int ev_idx = 0;
     double diff = 0.0;
     if (nf < 11 || name_end < 0 || f3 > 65535 || name_end - f3 > 65535) fl |= MC_RF_BADNUM | MC_RF_BADIDX;   // cannot happen for a kept line
-    else {
-        const uint8_t *lp = text + line;
-        uint32_t m_ev = 0u, m_md = 0u;
-        int n_ev = 0, n_md = 0;
-        const int teq = fast_tokens_equal8(load8_unaligned(lp + f2), load8_unaligned(lp + f9));
-        if (line + f10 + 16 < limit && teq >= 0 && fast_uint8(load8_unaligned(lp + f5), ev_idx) &&
-            fast_decimal8(load8_unaligned(lp + f6), m_ev, n_ev) && fast_decimal8(load8_unaligned(lp + f10), m_md, n_md)) {
-            const double ev = __ddiv_rn((double)m_ev, c_pow10[n_ev]), md = __ddiv_rn((double)m_md, c_pow10[n_md]);
-            diff = __ddiv_rn(rint(__dmul_rn(__dsub_rn(ev, md), 1e4)), 1e4);
-            if (teq) fl |= MC_RF_EQ;
-        } else {
-            const GlobalBytes t{text + line, limit - line};
-            ev_idx = 0;
-            parse_values(t, f2, f5, f6, f9, f10, ev_idx, diff, fl);
-        }
-    }
+    else mc_finish_values(text + line, limit - line, f2, f5, f6, f9, f10, ev_idx, diff, fl);
     r.name_off = (uint16_t)f3;
     r.name_len = (uint16_t)(name_end < 0 ? 0 : name_end - f3);
     r.event_idx = ev_idx;
@@ -287,19 +302,12 @@ __device__ __forceinline__ void mc_finish_record(const uint8_t *__restrict__ tex
 // Stage 1 parks the first 128 field-start bits of the recorded line (bit b: a column starts at line offset b) in the
 // raw record's event_idx / diff / name_off / name_len fields (pad bit 1: none).  With them the columns are located by
 // rank/select and only the bytes of the needed tokens are read: columns 3, 6, 7, 10, 11 and the end of the read name.
-// Falls back to the walk above when a needed column starts beyond the window or a token has an unusual shape.
-__device__ __forceinline__ int mc_nth_bit(uint32_t m, int j) {     // position of the j-th (0-based) set bit, j < popc(m)
-#pragma unroll
-    for (int t = 0; t < 6; ++t)
-        if (j > t) m &= m - 1u;
-    for (int t = 6; t < j; ++t) m &= m - 1u;
-    return __ffs(m) - 1;
-}
+// Falls back to the walk above when a needed column starts beyond the window.
 __device__ __forceinline__ void mc_finish_record_win(const uint8_t *__restrict__ text, int64_t limit, mc_record &r) {
     const uint32_t *rw = reinterpret_cast<const uint32_t *>(&r);
     const uint32_t W0 = rw[3], W1 = rw[4], W2 = rw[5], W3 = (rw[1] >> 16) | (rw[6] << 16);
     const int c0 = __popc(W0), c1 = c0 + __popc(W1), c2 = c1 + __popc(W2), c3 = c2 + __popc(W3);
-    const int64_t line = ((int64_t)r.line_hi << 32) | (int64_t)r.line_lo;
+    const int64_t line = mc_rec_line(r);
     if ((r.pad & 2u) || c3 < 11 || line + 160 >= limit) {            // no window / column 11 beyond it: walk the line
         r.pad = 0;
         mc_finish_record(text, limit, r);
@@ -330,7 +338,7 @@ __device__ __forceinline__ void mc_finish_record_win(const uint8_t *__restrict__
     int name_end;
     {
         const unsigned long long t8 = f4 >= 8 ? load8_unaligned(lp + f4 - 8) : 0ull;
-        const uint32_t nh = fin_gt20((uint32_t)(t8 >> 32)), nlw = fin_gt20((uint32_t)t8);     // 0x80 per non-whitespace byte
+        const uint32_t nh = gt20_msb((uint32_t)(t8 >> 32)), nlw = gt20_msb((uint32_t)t8);     // 0x80 per non-whitespace byte
         const int tw = nh ? (__clz(nh) >> 3) : nlw ? 4 + (__clz(nlw) >> 3) : 8;               // whitespace bytes right before column 5
         name_end = f4 - tw;
         if (tw == 8 || name_end <= f3) {
@@ -341,19 +349,7 @@ __device__ __forceinline__ void mc_finish_record_win(const uint8_t *__restrict__
     uint32_t fl = r.flags & ~MC_RF_RAW;
     int ev_idx = 0;
     double diff = 0.0;
-    uint32_t m_ev = 0u, m_md = 0u;
-    int n_ev = 0, n_md = 0;
-    const int teq = fast_tokens_equal8(load8_unaligned(lp + f2), load8_unaligned(lp + f9));
-    if (teq >= 0 && fast_uint8(load8_unaligned(lp + f5), ev_idx) && fast_decimal8(load8_unaligned(lp + f6), m_ev, n_ev) &&
-        fast_decimal8(load8_unaligned(lp + f10), m_md, n_md)) {
-        const double ev = __ddiv_rn((double)m_ev, c_pow10[n_ev]), md = __ddiv_rn((double)m_md, c_pow10[n_md]);
-        diff = __ddiv_rn(rint(__dmul_rn(__dsub_rn(ev, md), 1e4)), 1e4);
-        if (teq) fl |= MC_RF_EQ;
-    } else {
-        const GlobalBytes t{lp, limit - line};
-        ev_idx = 0;
-        parse_values(t, f2, f5, f6, f9, f10, ev_idx, diff, fl);
-    }
+    mc_finish_values(lp, limit - line, f2, f5, f6, f9, f10, ev_idx, diff, fl);
     r.name_off = (uint16_t)f3;
     r.name_len = (uint16_t)(name_end - f3);
     r.event_idx = ev_idx;

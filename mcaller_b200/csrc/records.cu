@@ -8,25 +8,19 @@ constexpr int SCAN_THREADS = 256;
 constexpr int SCAN_IPT = 8;
 constexpr int SCAN_BLOCK = SCAN_THREADS * SCAN_IPT;
 
-// ---- generic exclusive scan over uint32 (input may be strided) -----------------------------------------
-// the item count may live on the device (d_n != nullptr): n is then only the capacity the grid was sized for
-__device__ __forceinline__ int64_t dev_count(const unsigned long long *d_n, int64_t cap) {
-    if (!d_n) return cap;
-    const unsigned long long v = *d_n;
-    return v < (unsigned long long)cap ? (int64_t)v : cap;
-}
-
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_reduce(const uint32_t *__restrict__ in, int64_t stride, int64_t n_cap,
+// ---- generic exclusive scan over uint32 -----------------------------------------------------------------
+// the item count may live on the device (d_n != nullptr): n_cap is then only the capacity the grid was sized for
+__global__ void __launch_bounds__(SCAN_THREADS) k_scan_reduce(const uint32_t *__restrict__ in, int64_t n_cap,
                                                             const unsigned long long *__restrict__ d_n,
                                                             unsigned long long *__restrict__ block_sums) {
     __shared__ int s_warp[SCAN_THREADS / 32 + 1];
-    const int64_t n = dev_count(d_n, n_cap);
+    const int64_t n = d_n ? mc_dev_count(d_n, n_cap) : n_cap;
     const int64_t base = (int64_t)blockIdx.x * SCAN_BLOCK;
     unsigned long long acc = 0ull;
 #pragma unroll
     for (int j = 0; j < SCAN_IPT; ++j) {
         const int64_t i = base + (int64_t)j * SCAN_THREADS + threadIdx.x;
-        if (i < n) acc += in[i * stride];
+        if (i < n) acc += in[i];
     }
     // block reduce (64-bit)
     for (int d = 16; d > 0; d >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, d);
@@ -77,12 +71,12 @@ __global__ void __launch_bounds__(1024) k_scan_sums(unsigned long long *__restri
     if (threadIdx.x == 0 && d_total) *d_total = s_carry;
 }
 
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_down(const uint32_t *__restrict__ in, int64_t stride, int64_t n_cap,
+__global__ void __launch_bounds__(SCAN_THREADS) k_scan_down(const uint32_t *__restrict__ in, int64_t n_cap,
                                                           const unsigned long long *__restrict__ d_n,
                                                           const unsigned long long *__restrict__ block_sums,
                                                           uint32_t *__restrict__ out) {
     __shared__ int s_warp[SCAN_THREADS / 32 + 1];
-    const int64_t n = dev_count(d_n, n_cap);
+    const int64_t n = d_n ? mc_dev_count(d_n, n_cap) : n_cap;
     if ((int64_t)blockIdx.x * SCAN_BLOCK >= n) return;           // whole block beyond the count (block-uniform)
     // thread owns SCAN_IPT consecutive items so the scan order is the index order
     const int64_t base = (int64_t)blockIdx.x * SCAN_BLOCK + (int64_t)threadIdx.x * SCAN_IPT;
@@ -91,7 +85,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_down(const uint32_t *__re
 #pragma unroll
     for (int j = 0; j < SCAN_IPT; ++j) {
         const int64_t i = base + j;
-        v[j] = (i < n) ? in[i * stride] : 0u;
+        v[j] = (i < n) ? in[i] : 0u;
         sum += (int)v[j];
     }
     int total;
@@ -109,31 +103,22 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_down(const uint32_t *__re
 
 int64_t mc_exscan_ws_bytes(int64_t n) { return ((n + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * 8 + 256; }
 
-static int exscan_strided(const uint32_t *d_in, int64_t stride, uint32_t *d_out, int64_t n, const uint64_t *d_n, uint64_t *d_total,
-                          void *d_ws, cudaStream_t st) {
-    if (n <= 0) {
+int mc_exscan_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n_cap, const uint64_t *d_n, uint64_t *d_total, void *d_ws,
+                  cudaStream_t st) {
+    if (n_cap <= 0) {
         if (d_total) MC_CUDA_CHECK(cudaMemsetAsync(d_total, 0, 8, st));
         return MC_OK;
     }
-    const int64_t nb = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    const int64_t nb = (n_cap + SCAN_BLOCK - 1) / SCAN_BLOCK;
     unsigned long long *sums = reinterpret_cast<unsigned long long *>(d_ws);
     const unsigned long long *dn = reinterpret_cast<const unsigned long long *>(d_n);
-    k_scan_reduce<<<(unsigned)nb, SCAN_THREADS, 0, st>>>(d_in, stride, n, dn, sums);
+    k_scan_reduce<<<(unsigned)nb, SCAN_THREADS, 0, st>>>(d_in, n_cap, dn, sums);
     MC_LAUNCH_CHECK();
     k_scan_sums<<<1, 1024, 0, st>>>(sums, nb, reinterpret_cast<unsigned long long *>(d_total));
     MC_LAUNCH_CHECK();
-    k_scan_down<<<(unsigned)nb, SCAN_THREADS, 0, st>>>(d_in, stride, n, dn, sums, d_out);
+    k_scan_down<<<(unsigned)nb, SCAN_THREADS, 0, st>>>(d_in, n_cap, dn, sums, d_out);
     MC_LAUNCH_CHECK();
     return MC_OK;
-}
-
-int mc_exscan_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n, uint64_t *d_total, void *d_ws, cudaStream_t st) {
-    return exscan_strided(d_in, 1, d_out, n, nullptr, d_total, d_ws, st);
-}
-// n = capacity, the item count is read from d_n on the device (items beyond it count as zero)
-int mc_exscan_u32_dev(const uint32_t *d_in, uint32_t *d_out, int64_t n_cap, const uint64_t *d_n, uint64_t *d_total, void *d_ws,
-                      cudaStream_t st) {
-    return exscan_strided(d_in, 1, d_out, n_cap, d_n, d_total, d_ws, st);
 }
 
 // workspace layout used by the stages: [A: uint32 n][B: uint32 n][scan sums]
@@ -262,7 +247,7 @@ __global__ void __launch_bounds__(256, 4) k_gather_finish(const uint8_t *__restr
                         r.kbits_rev = (uint8_t)mc_kmer_bits(R.d_site_rev, g, R.k);
                     }
                 }
-                line = ((long long)r.line_hi << 32) | (long long)r.line_lo;
+                line = mc_rec_line(r);
                 span = (uint32_t)r.name_off | ((uint32_t)r.name_len << 16);
             }
             // read name against the previous record of the run (same read <=> equal bytes, extract_contexts.py:161)
@@ -296,13 +281,11 @@ __global__ void __launch_bounds__(256, 4) k_gather_finish(const uint8_t *__restr
     }
 }
 
-__device__ __forceinline__ int64_t rec_line(const mc_record &r) { return ((int64_t)r.line_hi << 32) | (int64_t)r.line_lo; }
-
 // ---- stage 3: read segmentation ----------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_seg_flags(const uint8_t *__restrict__ text, mc_record *__restrict__ rec, int64_t n_cap,
                                                   const unsigned long long *__restrict__ d_n, uint32_t *__restrict__ flags,
                                                   const uint32_t *__restrict__ known) {
-    const int64_t n = dev_count(d_n, n_cap);
+    const int64_t n = mc_dev_count(d_n, n_cap);
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     if (known) {                                                  // stage 2 left the answer for all but the first record of a run
@@ -320,7 +303,7 @@ __global__ void __launch_bounds__(256) k_seg_flags(const uint8_t *__restrict__ t
         if (i > 0) {
             const mc_record a = rec[i - 1];
             if (a.name_len == b.name_len)
-                f = bytes_differ(text + rec_line(a) + a.name_off, text + rec_line(b) + b.name_off, a.name_len) ? 1u : 0u;
+                f = bytes_differ(text + mc_rec_line(a) + a.name_off, text + mc_rec_line(b) + b.name_off, a.name_len) ? 1u : 0u;
         }
         rec[i].flags = (uint8_t)(b.flags | MC_RF_SEGKNOWN | (f ? MC_RF_NEWREAD : 0u));
     }
@@ -334,13 +317,13 @@ __global__ void __launch_bounds__(256) k_seg_fix(const uint8_t *__restrict__ tex
     const int64_t run = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (run >= n_runs) return;
     const uint32_t i = run_first[run];
-    if (i == 0xFFFFFFFFu || (int64_t)i >= dev_count(d_n, n_cap)) return;
+    if (i == 0xFFFFFFFFu || (int64_t)i >= mc_dev_count(d_n, n_cap)) return;
     uint32_t f = 1u;
     const mc_record b = rec[i];
     if (i > 0u) {
         const mc_record a = rec[i - 1];
         if (a.name_len == b.name_len)
-            f = bytes_differ(text + rec_line(a) + a.name_off, text + rec_line(b) + b.name_off, a.name_len) ? 1u : 0u;
+            f = bytes_differ(text + mc_rec_line(a) + a.name_off, text + mc_rec_line(b) + b.name_off, a.name_len) ? 1u : 0u;
     }
     rec[i].flags = (uint8_t)(b.flags | MC_RF_SEGKNOWN | (f ? MC_RF_NEWREAD : 0u));
     flags[i] = f;
@@ -349,7 +332,7 @@ __global__ void __launch_bounds__(256) k_seg_fix(const uint8_t *__restrict__ tex
 __global__ void __launch_bounds__(256) k_seg_starts(const uint32_t *__restrict__ flags, const uint32_t *__restrict__ excl, int64_t n_cap,
                                                    const unsigned long long *__restrict__ d_n, uint32_t *__restrict__ seg_start,
                                                    const unsigned long long *__restrict__ d_nseg) {
-    const int64_t n = dev_count(d_n, n_cap);
+    const int64_t n = mc_dev_count(d_n, n_cap);
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n && flags[i]) seg_start[excl[i]] = (uint32_t)i;
     if (i == 0) seg_start[*d_nseg] = (uint32_t)n;
@@ -361,28 +344,17 @@ __global__ void __launch_bounds__(256) k_seg_quality(const uint8_t *__restrict__
                                                     const unsigned long long *__restrict__ d_nseg,
                                                     const mc_qual_entry *__restrict__ table, unsigned long long mask,
                                                     double *__restrict__ seg_qual, unsigned long long *__restrict__ d_err) {
-    const int64_t n_seg = dev_count(d_nseg, seg_cap);
+    const int64_t n_seg = mc_dev_count(d_nseg, seg_cap);
     const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_seg) return;
     const mc_record r = rec[seg_start[s]];
-    const uint8_t *p = text + rec_line(r) + r.name_off;
-    // key = name.split(':')[0].split('_')[0]   (read_qual.py:11-12 / extract_contexts.py:166)
-    unsigned long long h = 14695981039346656037ull, h2 = 0x84222325cbf29ce4ull;
-    int len = 0;
-    for (; len < r.name_len; ++len) {
-        const unsigned c = __ldg(p + len);
-        if (c == ':' || c == '_') break;
-        h = (h ^ c) * 1099511628211ull;
-        h2 = (h2 ^ c) * 1099511628211ull;
-    }
-    if (h == 0ull) h = 1ull;
-    const uint32_t check = (uint32_t)(h2 >> 32);
+    const mc_read_key key = mc_read_key_of(text + mc_rec_line(r) + r.name_off, r.name_len);
     double q = __longlong_as_double(0x7ff8000000000000ll);   // NaN = missing
-    unsigned long long slot = h & mask;
+    unsigned long long slot = key.hash & mask;
     for (unsigned long long probe = 0; probe <= mask; ++probe) {
         const mc_qual_entry e = table[slot];
         if (e.hash == 0ull) break;
-        if (e.hash == h && e.check == check && e.len == (uint32_t)len) { q = e.qual; break; }
+        if (e.hash == key.hash && e.check == key.check && e.len == key.len) { q = e.qual; break; }
         slot = (slot + 1) & mask;
     }
     if (q != q) atomicAdd(d_err, 1ull);
@@ -409,7 +381,7 @@ extern "C" int mc_order_records(const uint8_t *d_text, int64_t nbytes, const mc_
     k_run_resolve<<<(unsigned)((n_runs + 255) / 256), 256, 0, st>>>(d_run_tab, n_runs, cnt, reinterpret_cast<const unsigned long long *>(d_scan_counters),
                                                                    (unsigned long long)rec_in_cap);
     MC_LAUNCH_CHECK();
-    int rc = mc_exscan_u32(cnt, dst, n_runs + 1, d_n_out, ws_s(d_ws, n_runs + 1), st);     // entry n_runs (count 0) = the total
+    int rc = mc_exscan_u32(cnt, dst, n_runs + 1, nullptr, d_n_out, ws_s(d_ws, n_runs + 1), st);     // entry n_runs (count 0) = the total
     if (rc) return rc;
     int64_t gf_blocks = (n_runs * 32 + 255) / 256;
     {
@@ -447,7 +419,7 @@ extern "C" int mc_segment_reads(const uint8_t *d_text, mc_record *d_rec, const u
         k_seg_flags<<<nb, 256, 0, st>>>(d_text, d_rec, rec_cap, dn, flags, nullptr);
     }
     MC_LAUNCH_CHECK();
-    int rc = mc_exscan_u32_dev(flags, excl, rec_cap, d_n_records, d_nseg, ws_s(d_ws, rec_cap), st);
+    int rc = mc_exscan_u32(flags, excl, rec_cap, d_n_records, d_nseg, ws_s(d_ws, rec_cap), st);
     if (rc) return rc;
     k_seg_starts<<<nb, 256, 0, st>>>(flags, excl, rec_cap, dn, d_seg_start, reinterpret_cast<const unsigned long long *>(d_nseg));
     MC_LAUNCH_CHECK();

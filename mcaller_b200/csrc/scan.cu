@@ -102,9 +102,8 @@ __device__ __forceinline__ bool mbar_wait(unsigned long long *bar, uint32_t pari
 }
 
 // ---- byte classification ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t gt20_msb(uint32_t w) { return (((w & 0x7f7f7f7fu) + 0x5f5f5f5fu) | w) & 0x80808080u; }
-// 8 msb-form words (0x80 per flagged byte) -> 32 flag bits in byte order.  IDP.4A sums 0x80 * weight per byte: two
-// words fill bits 7..14 of one accumulator.
+// 8 msb-form words (0x80 per flagged byte) -> 32 flag bits in byte order, as pack16 does for 4
+// (not two pack16 calls: their OR form costs k_scan about 40 more instructions than this sum)
 __device__ __forceinline__ uint32_t pack32(uint32_t m0, uint32_t m1, uint32_t m2, uint32_t m3, uint32_t m4, uint32_t m5,
                                            uint32_t m6, uint32_t m7) {
     const uint32_t lo = 0x08040201u, hi = 0x80402010u;
@@ -141,13 +140,6 @@ __device__ __forceinline__ int next_bit(const uint32_t *m, int q) {
 }
 
 // ---- field location: 160-bit window of field-start bits aligned at the line start, branch-free rank/select -------------
-__device__ __forceinline__ int nth_bit(uint32_t m, int j) {     // position of the j-th (0-based) set bit, j < popc(m)
-#pragma unroll
-    for (int t = 0; t < 6; ++t)
-        if (j > t) m &= m - 1u;
-    for (int t = 6; t < j; ++t) m &= m - 1u;                     // words with more than 7 field starts: rare
-    return __ffs(m) - 1;
-}
 template <bool WANT3>
 __device__ __forceinline__ void line_fields(const WarpSmem &S, int s, int &f0, int &f1, int &f9, int &f11, int &f3) {
     const int w0 = s >> 5, sh = s & 31;
@@ -207,10 +199,6 @@ __device__ __forceinline__ unsigned long long load8(const uint8_t *text, int q) 
 
 // position column decoded from its first 8 bytes in registers: up to 7 digits and the byte that ends them.
 // Returns 1 (pos set), 0 (not a number / not followed by whitespace) or -1 (8 or more digits: take the byte loop).
-__device__ __forceinline__ uint32_t conv4(uint32_t h) {            // 4 digit values, most significant in byte 0 -> 0..9999
-    const uint32_t t = ((h * 2561u) >> 8) & 0x00ff00ffu;
-    return (t * 6553601u) >> 16;
-}
 __device__ __forceinline__ int parse_pos8(unsigned long long k8, int &pos) {
     const uint32_t lo = (uint32_t)k8, hi = (uint32_t)(k8 >> 32);
     const uint32_t xl = lo ^ 0x30303030u, xh = hi ^ 0x30303030u;
@@ -248,7 +236,8 @@ __device__ __forceinline__ bool token_is(const uint8_t *text, int q, int len, co
     for (int j = 0; 8 * j < len; ++j) eq = eq && low_bytes(load8(text, q + 8 * j), len - 8 * j) == key[j];
     return eq;
 }
-__device__ __forceinline__ bool tokens_equal(const uint8_t *text, int qa, int qb, int len) {
+// the `len` bytes at qa equal the `len` bytes at qb
+__device__ __forceinline__ bool spans_equal(const uint8_t *text, int qa, int qb, int len) {
     bool eq = true;
     for (int j = 0; 8 * j < len; ++j) eq = eq && low_bytes(load8(text, qa + 8 * j) ^ load8(text, qb + 8 * j), len - 8 * j) == 0ull;
     return eq;
@@ -733,7 +722,7 @@ k_scan(const uint8_t *__restrict__ d_text, int64_t nbytes, int64_t text_limit16,
                 bool same = false;
                 if (valid && nlen > 0) {
                     if (lane == 0) same = nlen == rname_len && token_is(text, nq, nlen, S.rname);
-                    else same = nlen == plen && tokens_equal(text, nq, pq, nlen);
+                    else same = nlen == plen && spans_equal(text, nq, pq, nlen);
                 }
                 const uint32_t pass_m = n_pass >= 32 ? 0xFFFFFFFFu : ((1u << n_pass) - 1u);
                 new_m = __ballot_sync(0xffffffffu, !same) & pass_m;

@@ -71,8 +71,6 @@ __device__ __forceinline__ void cnt_clear(Counts &q, int c) {
 }
 __device__ __forceinline__ int map_get(uint32_t mp, int c) { return (int)((mp >> (4 * c)) & 0xFu); }
 
-__device__ __forceinline__ int64_t rec_line(const mc_record &r) { return ((int64_t)r.line_hi << 32) | (int64_t)r.line_lo; }
-
 __device__ __forceinline__ mc_record load_rec(const mc_record *p) {
     mc_record r;
     const uint4 *s = reinterpret_cast<const uint4 *>(p);
@@ -359,7 +357,7 @@ k_windows(const mc_record *__restrict__ rec, int64_t rec_cap, const unsigned lon
             if (out_pos < call_cap) {
                 mc_call &o = calls[out_pos];
                 const mc_record nr = load_rec(rec + name_rec);
-                o.read_off = rec_line(nr) + nr.name_off;
+                o.read_off = mc_rec_line(nr) + nr.name_off;
                 o.read_len = nr.name_len;
                 o.prob = 0.0;
                 o.mpos = mpos;
@@ -424,7 +422,7 @@ k_windows(const mc_record *__restrict__ rec, int64_t rec_cap, const unsigned lon
             if (out_pos < call_cap) {
                 mc_call &o = calls[out_pos];
                 const mc_record nr = load_rec(rec + name_rec);
-                o.read_off = rec_line(nr) + nr.name_off;
+                o.read_off = mc_rec_line(nr) + nr.name_off;
                 o.read_len = nr.name_len;
                 o.prob = 0.0;
                 for (int c = 0; c <= MC_MAXK; ++c) o.feat[c] = 0.0;
@@ -623,7 +621,7 @@ extern "C" int mc_build_windows(const mc_record *d_rec, const uint64_t *d_n_reco
                                                           *ref, skip_thresh, qual_thresh, two_models, d_calls,
                                                           (unsigned long long)call_cap, unit_cnt, blk_tot, nullptr, tags, spill);
     MC_LAUNCH_CHECK();
-    int rc = mc_exscan_u32(blk_tot, blk_off, nb, d_ncalls, scan_ws, st);
+    int rc = mc_exscan_u32(blk_tot, blk_off, nb, nullptr, d_ncalls, scan_ws, st);
     if (rc) return rc;
     k_windows<true><<<(unsigned)nb, WIN_THREADS, rec_bytes + diff_bytes, st>>>(d_rec, rec_cap, dn, d_seg_start, seg_cap, ds, d_seg_qual, first_idx,
                                                                   first_ind, *ref, skip_thresh, qual_thresh, two_models, d_calls,

@@ -143,8 +143,9 @@ def test_golden_inputs_are_stable(tmp_path):
         assert hashlib.sha256(open(inp["tsv"], "rb").read()).hexdigest() == gold["tsv_sha256"]
 
 
-def test_c_abi_exports_match_header():
-    """Every function declared in include/mcaller_b200.h is exported by the built library and bound in _lib."""
+def test_c_abi_v3_exports_match_header():
+    """ABI version 3: every function declared in include/mcaller_b200.h is exported by the built library and bound in
+    _lib, and the unused mc_diffs_aggregate that version 2 exported is gone."""
     from mcaller_b200 import _lib, build
     build.build()
     hdr = open(os.path.join(os.path.dirname(gc.GOLD), "..", "include", "mcaller_b200.h")).read()
@@ -154,7 +155,8 @@ def test_c_abi_exports_match_header():
     for fn in declared:
         assert hasattr(lib, fn), fn
     assert declared == set(_lib.EXPORTS)
-    assert lib.mc_version() == _lib.MC_ABI_VERSION == 2
+    assert not hasattr(lib, "mc_diffs_aggregate")
+    assert lib.mc_version() == _lib.MC_ABI_VERSION == 3
     assert lib.mc_num_tiles(1) == 1 and lib.mc_num_tiles(3840) == 1 and lib.mc_num_tiles(3841) == 2
     assert lib.mc_workspace_bytes(1000) > 8000
 
