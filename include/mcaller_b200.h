@@ -434,6 +434,39 @@ int mc_fastq_index(const uint8_t *d_text, int64_t nbytes, uint32_t *d_tile_cnt, 
 int mc_fastq_quality(const uint8_t *d_text, int64_t nbytes, const uint64_t *d_line_start, int64_t n_lines, mc_qual_entry *d_table,
                      int64_t table_size, uint32_t *d_owner, double *d_rec_mean, uint64_t *d_stats, void *stream);
 
+/*
+ * MLP training (mCaller --train -c NN): scikit-learn 1.9 MLPClassifier(hidden_layer_sizes=MC_TRAIN_HIDDEN,
+ * activation='tanh', solver='adam', batch_size='auto', shuffle=True).fit on a binary target, float64, one CTA per job.
+ * The caller draws the initial parameters and every epoch's sample order from numpy's RandomState(seed) as scikit-learn
+ * does, writes the parameters to d_w (W0 [d][100] row-major, W1 [100], c0 [100], c1 [1]; n_params = 102 d + 101) and the
+ * job array to device memory, and calls mc_mlp_train_init once (Adam moments zeroed, state reset).  Each
+ * mc_mlp_train_epochs call then runs up to `epochs` epochs of every job not yet stopped: epoch e of job j visits the rows
+ * d_idx[idx_off + e*n .. + n) (indices into d_x / d_y) in batches of min(MC_TRAIN_BATCH, n), the last one possibly short.
+ * After an epoch the kernel appends the epoch loss to d_loss_curve and applies the no-improvement rule (loss > best - tol
+ * counts; stop when the count exceeds n_iter_no_change, stopped = 1) and the iteration limit (stopped = 2).  The state
+ * stays in d_w and the job array between calls, so the caller can draw the next epochs' orders while a call runs, and
+ * read `stopped` back after it.  Requirements: 1 <= d <= MC_MAXK + 1, n >= 1; d_idx entries index valid rows for every
+ * epoch of the call (also the epochs of a job that stops early).
+ */
+#define MC_TRAIN_HIDDEN 100
+#define MC_TRAIN_BATCH 200
+typedef struct mc_train_job {
+    const double *d_x;           /* [rows][d] features, row-major */
+    const double *d_y;           /* [rows] target, 0.0 or 1.0 */
+    double *d_w;                 /* [3][n_params]: parameters (in: initial, out: fitted), Adam m, Adam v */
+    double *d_loss_curve;        /* [max_iter] epoch losses (scikit-learn's loss_curve_) */
+    int64_t idx_off;             /* this job's [epochs][n] sample orders in the d_idx of each call */
+    int32_t n, d;                /* training rows, features */
+    int32_t max_iter, n_iter_no_change;
+    double alpha, lr, tol;
+    /* kept by the kernels */
+    double best_loss;
+    int32_t n_iter, no_improve, stopped, pad;
+} mc_train_job;                  /* 104 bytes */
+
+int mc_mlp_train_init(mc_train_job *d_jobs, int32_t n_jobs, void *stream);
+int mc_mlp_train_epochs(mc_train_job *d_jobs, int32_t n_jobs, const int32_t *d_idx, int32_t epochs, void *stream);
+
 /* ---- synthetic eventalign generator (bench / test tooling; bit-identical to mcaller_b200/synth.py) ---- */
 typedef struct mc_synth_spec {
     uint64_t seed;

@@ -61,6 +61,15 @@ class LocusEntry(C.Structure):
     _fields_ = [("hash", C.c_uint64), ("first_off", C.c_uint64), ("check", C.c_uint64), ("depth", C.c_uint32), ("meth", C.c_uint32)]
 
 
+class TrainJob(C.Structure):
+    _fields_ = [("d_x", C.c_void_p), ("d_y", C.c_void_p), ("d_w", C.c_void_p), ("d_loss_curve", C.c_void_p), ("idx_off", C.c_int64),
+                ("n", C.c_int32), ("d", C.c_int32), ("max_iter", C.c_int32), ("n_iter_no_change", C.c_int32), ("alpha", C.c_double),
+                ("lr", C.c_double), ("tol", C.c_double), ("best_loss", C.c_double), ("n_iter", C.c_int32), ("no_improve", C.c_int32),
+                ("stopped", C.c_int32), ("pad", C.c_int32)]
+
+
+MC_TRAIN_HIDDEN, MC_TRAIN_BATCH = 100, 200
+
 CARRY_BYTES = 192          # sizeof(mc_carry): the row (128 B), valid, first_kept_contig, chunk count, padding
 
 QUAL_DTYPE = np.dtype([("hash", "<u8"), ("check", "<u4"), ("len", "<u4"), ("qual", "<f8")])
@@ -136,6 +145,10 @@ _PROTOS = {
     "mc_diffs_rehash": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "mc_diffs_rows": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
                                 C.c_void_p]),
+    # d_jobs, n_jobs, stream
+    "mc_mlp_train_init": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
+    # d_jobs, n_jobs, d_idx, epochs, stream
+    "mc_mlp_train_epochs": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "mc_diffs_colstats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
 }

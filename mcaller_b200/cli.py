@@ -2,6 +2,7 @@
 
     python -m mcaller_b200.cli mCaller  -m GATC -r ref.fa -e x.eventalign.tsv -f x.fastq -d model.pkl -b A
     python -m mcaller_b200.cli make_bed -f x.eventalign.diffs.6 -d 15 -t 0.5
+    python -m mcaller_b200.cli mCaller --train -p labelled_positions.txt -r ref.fa -e x.eventalign.tsv -f x.fastq -b A -c NN
 
 The reference's own mCaller.py / make_bed.py can be used unchanged instead (INTEGRATION.md); these entry points exist
 so the path can be run where the reference checkout is absent.  `-t N` splits the TSV into N read-aligned byte ranges
@@ -43,9 +44,8 @@ def mcaller_main(argv=None):
     p.add_argument("--bed_control", action="store_true")
     p.add_argument("--bed_gff", action="store_true")
     p.add_argument("--bed_ref", type=str)
+    p.add_argument("--seed", type=int, default=0, help="random_state of the training's balancing, folds and fits")
     a = p.parse_args(argv)
-    if a.train or a.training_tsv:
-        raise NotImplementedError("training stays with the reference (out of scope of the accelerated path)")
     if a.base == "A":
         mod = "m6A"
     elif a.base == "C":
@@ -53,6 +53,8 @@ def mcaller_main(argv=None):
     else:
         print("classification only available for A or C bases so far")
         return 0
+    if a.train or a.training_tsv:
+        return _train_main(p, a, mod)
     modelfile = a.modelfile or (os.path.dirname(os.path.realpath(sys.argv[0])) + "/model_" + a.classifier + "_" + str(a.num_variables) + "_" + mod + ".pkl")
     assert os.path.isfile(modelfile), "model file not found at " + modelfile
     base = a.motif if (a.motif and len(a.motif) == 1) else a.base
@@ -79,6 +81,66 @@ def mcaller_main(argv=None):
                             endline=end, train=False, base=base, motif=a.motif, positions_list=a.positions)
     print("Finished extracting signals")
     multigpu.merge_outputs(a.tsv, k, len(ranges))
+    return 0
+
+
+def _train_main(p, a, mod):
+    """--train: labelled windows -> `<prefix>.diffs.<k>.train` -> model fit -> pickle; --training_tsv: fit on an existing
+    `.train` file (INTEGRATION.md, "Training")."""
+    import pickle
+    from . import extract_contexts as ec, multigpu, read_qual, refmark, train as tr
+    if a.classifier in ("RF", "LR"):
+        raise NotImplementedError("-c %s training is not supported: the reference's RandomForest / LogisticRegression settings "
+                                  "are rejected by scikit-learn 1.9" % a.classifier)
+    if a.classifier not in ("NN", "NBC"):
+        p.error("-c must be NN, NBC, RF or LR")
+    if a.plot_training:
+        raise NotImplementedError("--plot_training: training plots are not produced")
+    if a.gpus:
+        raise NotImplementedError("--train runs in one process; --gpus applies to calling only")
+    k = a.num_variables
+    out = a.modelfile or "model_%s_%d_%s.pkl" % (a.classifier, k, mod)
+    if a.training_tsv:
+        assert os.path.isfile(a.training_tsv), "training file not found at " + a.training_tsv
+        sites, x, labels, ctxs = tr.read_train_tsv(a.training_tsv)
+        keys = tr.keys_from_contexts(ctxs, a.base, k)
+    else:
+        if not a.positions:
+            p.error("--train needs labelled positions (-p, 4th column: label), not a motif")
+        pos_label = {}
+        with open(a.positions) as fh:
+            for ln in fh:
+                f = ln.split()
+                if not f:
+                    continue
+                if len(f) < 4:
+                    p.error("--train: %s has no label column (contig, position, strand, label)" % a.positions)
+                pos_label[(f[0], int(f[1]), f[2])] = f[3]
+        assert a.skip_thresh < k / 2, "too many skips with only " + str(k) + " variables - try < half"
+        assert os.path.isfile(a.fastq), "fastq file not found at " + a.fastq
+        read2qual = read_qual.extract_read_quality_device(a.fastq)
+        print("%d contigs" % len(refmark.read_fasta(a.reference)))
+        print("%d threads" % a.threads)
+        ranges = multigpu.byte_ranges(os.path.getsize(a.tsv), max(1, a.threads))
+        keys = []
+        for start, end in ranges:
+            tmp = ec.diffs_name(a.tsv, k, start, train=True)
+            if os.path.exists(tmp):
+                os.remove(tmp)
+            run = ec.RangeRun(a.tsv, a.reference, read2qual, k, a.skip_thresh, a.qual_thresh, None, start, endline=end, train=True,
+                              pos_label=pos_label, base=a.base, positions_list=a.positions)
+            run.stream()
+            run.close_by_probe()
+            run.print_counters()
+            keys += run.fmt.keys
+        print("Finished extracting signals")
+        sites, x, labels, _ = tr.read_train_tsv(multigpu.merge_outputs(a.tsv, k, len(ranges), train=True))
+        if len(keys) != len(labels):
+            raise RuntimeError("%d rows written, %d model keys" % (len(labels), len(keys)))
+    model = tr.train(tr.TrainRows(sites, x, labels, keys), a.classifier, a.seed, mod, ["MG", "MH"] if a.base == "A" else ["general"])
+    with open(out, "wb") as fh:
+        pickle.dump(model, fh)
+    print("model written to %s" % out)
     return 0
 
 

@@ -22,7 +22,7 @@ extern "C" int mc_read_u64(const uint64_t *d_src, int64_t n, uint64_t *h_dst, vo
 }
 
 // struct sizes, so bindings in other languages can verify their layout (0 record, 1 call, 2 refindex, 3 model,
-// 4 qual entry, 5 synth spec, 6 locus entry)
+// 4 qual entry, 5 synth spec, 6 locus entry, 7 diffs row, 8 carry, 9 training job)
 extern "C" int mc_sizeof(int what) {
     switch (what) {
         case 0: return (int)sizeof(mc_record);
@@ -34,6 +34,7 @@ extern "C" int mc_sizeof(int what) {
         case 6: return (int)sizeof(mc_locus_entry);
         case 7: return (int)sizeof(mc_diffs_row);
         case 8: return (int)sizeof(mc_carry);
+        case 9: return (int)sizeof(mc_train_job);
         default: return -1;
     }
 }

@@ -13,58 +13,17 @@ namespace {
 constexpr int MAX_WIDTH = 512;     // widest MLP layer supported
 constexpr int WARPS = 8;
 
-__device__ __forceinline__ double expit(double x) { return x < 0.0 ? exp(x) / (1.0 + exp(x)) : 1.0 / (1.0 + exp(-x)); }
-
-// tanh(x) = sign(x) (1 - t) / (1 + t), t = exp(-2|x|), without branches: n = rint(y log2 e), r = y - n ln 2 (two-step), exp(r) by
-// its degree-13 Taylor polynomial on |r| <= ln2 / 2 (remainder < 5e-18), 2^n through the exponent field.  Absolute error
-// ~2e-16 -- the hidden activations feed a dot product whose result only has to match scikit-learn's float64 to 1e-12 --
-// at a third of the instructions of the library routine and with every lane on the same path (the float64 tanh was 55 % of
-// k_mlp_1hidden's instructions at 14 of 32 lanes active).
-__device__ __forceinline__ double mc_tanh(double x) {
-    double y = -2.0 * fabs(x);
-    y = fmax(y, -80.0);                                        // t < 2e-35: the quotient is 1 to the last bit
-    const double n = rint(y * 1.4426950408889634074);
-    double r = fma(n, -6.93147180369123816490e-01, y);
-    r = fma(n, -1.90821492927058770002e-10, r);
-    double p = 1.6059043836821613e-10;                         // 1/13!
-    p = fma(p, r, 2.0876756987868100e-09);                     // 1/12!
-    p = fma(p, r, 2.5052108385441720e-08);                     // 1/11!
-    p = fma(p, r, 2.7557319223985890e-07);                     // 1/10!
-    p = fma(p, r, 2.7557319223985893e-06);                     // 1/9!
-    p = fma(p, r, 2.4801587301587302e-05);                     // 1/8!
-    p = fma(p, r, 1.9841269841269841e-04);                     // 1/7!
-    p = fma(p, r, 1.3888888888888889e-03);                     // 1/6!
-    p = fma(p, r, 8.3333333333333332e-03);                     // 1/5!
-    p = fma(p, r, 4.1666666666666664e-02);                     // 1/4!
-    p = fma(p, r, 1.6666666666666666e-01);                     // 1/3!
-    p = fma(p, r, 0.5);
-    p = fma(p, r, 1.0);
-    p = fma(p, r, 1.0);
-    const double t = p * __longlong_as_double((long long)(1023 + (int)n) << 52);
-    // (1 - t) / (1 + t) without the division routine: 1 + t lies in [1, 2], a single-precision reciprocal is refined by two
-    // Newton steps (24 -> 48 -> 96 bits) and the quotient gets one residual correction (<= 1 ulp)
-    const double d = 1.0 + t, u = 1.0 - t;
-    double rc = (double)__frcp_rn((float)d);
-    double e = fma(-d, rc, 1.0);
-    rc = fma(rc, e, rc);
-    e = fma(-d, rc, 1.0);
-    rc = fma(rc, e, rc);
-    double q = u * rc;
-    q = fma(fma(-d, q, u), rc, q);
-    return copysign(q, x);
-}
-
 __device__ __forceinline__ double activate(double v, int act) {
     switch (act) {
         case MC_ACT_TANH: return mc_tanh(v);
-        case MC_ACT_LOGISTIC: return expit(v);
+        case MC_ACT_LOGISTIC: return mc_expit(v);
         case MC_ACT_RELU: return v > 0.0 ? v : 0.0;
         default: return v;
     }
 }
 
 // sklearn MLPClassifier._forward_pass_fast (neural_network/_multilayer_perceptron.py) for a binary classifier:
-// hidden activations, logistic output, P(class 1) = expit(z).
+// hidden activations, logistic output, P(class 1) = mc_expit(z).
 // Persistent warps: a block stages the weights and intercepts of both models in shared memory once (7-100-1: 7.2 KB per
 // model) and its warps then stride over the calls, so the inner loops read nothing but shared memory; the features of a
 // warp's next call are fetched while the current one is evaluated.  STAGED = false (models too wide for shared memory)
@@ -154,7 +113,7 @@ k_mlp(mc_call *__restrict__ calls, int64_t n_cap, const unsigned long long *__re
                 w += (size_t)ni * no;
                 bi += no;
             }
-            const double out = expit(x[0]);
+            const double out = mc_expit(x[0]);
             __syncwarp();
             if (lane == 0) {
                 mc_call &c = calls[i];
@@ -254,7 +213,7 @@ k_mlp_1hidden(mc_call *__restrict__ calls, const uint32_t *__restrict__ idx, con
         out += __shfl_xor_sync(0xffffffffu, out, 1);
         out += __shfl_xor_sync(0xffffffffu, out, 2);
         if (ks >= 0 && g == 0) {
-            const double p = expit(out + b1[0]);
+            const double p = mc_expit(out + b1[0]);
             mc_call &c = calls[i];
             c.prob = p;
             c.label = (uint8_t)(p >= 0.5);
@@ -262,7 +221,7 @@ k_mlp_1hidden(mc_call *__restrict__ calls, const uint32_t *__restrict__ idx, con
     }
 }
 
-// LogisticRegression.predict_proba (binary): expit(x.w + b); GaussianNB.predict_proba: exp(jll_1 - logsumexp(jll))
+// LogisticRegression.predict_proba (binary): mc_expit(x.w + b); GaussianNB.predict_proba: exp(jll_1 - logsumexp(jll))
 __global__ void __launch_bounds__(256) k_linear(mc_call *__restrict__ calls, int64_t n_cap, const unsigned long long *__restrict__ d_n,
                                                mc_model m0, mc_model m1) {
     const int64_t n = mc_dev_count(d_n, n_cap);
@@ -275,7 +234,7 @@ __global__ void __launch_bounds__(256) k_linear(mc_call *__restrict__ calls, int
     if (m.kind == MC_LR) {
         double z = __ldg(m.d_biases);
         for (int k = 0; k < m.n_in; ++k) z += c.feat[k] * __ldg(m.d_weights + k);
-        p = expit(z);
+        p = mc_expit(z);
     } else {
         const double *theta = m.d_weights, *var = m.d_weights + 2 * m.n_in;
         double jll[2];

@@ -201,9 +201,10 @@ class _RowFormatter(object):
     and the signal / context matrices train_model takes.  The carried window's read name and the counters are the
     TextSink's (`sink`)."""
 
-    def __init__(self, refindex, k, pos_label, sink):
-        self.ref, self.k, self.pos_label, self.sink = refindex, k, pos_label, sink
+    def __init__(self, refindex, k, pos_label, sink, two_models=False):
+        self.ref, self.k, self.pos_label, self.sink, self.two_models = refindex, k, pos_label, sink, two_models
         self.signals, self.contexts = {}, {}
+        self.keys = []                 # model key of each row written, from the window builder's model_sel (mCaller --train)
 
     def _row(self, c, read):
         k = self.k
@@ -218,6 +219,7 @@ class _RowFormatter(object):
         label = self.pos_label[(chrom, mpos, strand(rev))]
         self.signals.setdefault("general", {}).setdefault(label, []).append([float(x) for x in feat[:k + 1]])
         self.contexts.setdefault("general", {}).setdefault(label, []).append(ctx)
+        self.keys.append(("MG" if c["model_sel"] else "MH") if self.two_models else "general")
         return [chrom, read.decode(), str(mpos), ctx, ",".join(feats), strand(rev), label]
 
     def consume(self, calls, host_text_ptr, n_segments):
@@ -271,7 +273,7 @@ class RangeRun(object):
         except refmark.MarkError as e:
             print(str(e) + " - quitting thread now")
             raise ReferenceAbort(str(e))
-        dm, two = None, False
+        dm, two = None, train and base == "A"        # training -b A: rows get the MG/MH choice of a two-model pickle
         self.tsv_output = diffs_name(tsv_input, k, startline, train)
         if not train:
             model = _models.load_model_file(modelfile)
@@ -288,7 +290,7 @@ class RangeRun(object):
         if row_base:
             self.eng.reset_stream_state(row_base)
         self.sink = _stream.TextSink(self.ref, k, base, with_prob=dm is not None)
-        self.fmt = _RowFormatter(self.ref, k, pos_label, self.sink) if train else None
+        self.fmt = _RowFormatter(self.ref, k, pos_label, self.sink, two_models=two) if train else None
         self.fsize = os.path.getsize(tsv_input)
         if endline is None:
             endline = self.fsize

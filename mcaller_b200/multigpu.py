@@ -93,14 +93,15 @@ def ec_tmp_name(tsv, k, start):
     return diffs_name(tsv, k, start)
 
 
-def merge_outputs(tsv, k, world):
-    """Ranges do not overlap: concatenation in offset order == the -t 1 `.diffs.<k>` (no sort | uniq as in mCaller.py:103-107)."""
+def merge_outputs(tsv, k, world, train=False):
+    """Ranges do not overlap: concatenation in offset order == the -t 1 `.diffs.<k>` (no sort | uniq as in mCaller.py:103-107);
+    with `train`, the `.diffs.<k>.train` of a training run."""
     from .extract_contexts import diffs_name
     size = os.path.getsize(tsv)
-    out = diffs_name(tsv, k)
+    out = diffs_name(tsv, k, train=train)
     with open(out, "wb") as dst:
         for start, _ in byte_ranges(size, world):
-            tmp = ec_tmp_name(tsv, k, start)
+            tmp = diffs_name(tsv, k, start, train)
             if os.path.exists(tmp):
                 with open(tmp, "rb") as src:
                     while True:
