@@ -317,7 +317,9 @@ int mc_carry_close(mc_carry *d_carry, int closing_contig, const int64_t *d_next_
 /*
  * Stage 6 -- classifier: model[key].predict_proba([x])[0][1] and the 0.5 label threshold
  * (extract_contexts.py:195-207) for every MC_CALL row; float64 arithmetic.  models[0] = 'MH'/'general',
- * models[1] = 'MG' (only read when a row has model_sel == 1).  d_nrows[0] (device) rows, row_cap >= it.  d_ws: scratch of
+ * models[1] = 'MG' (used for rows with model_sel == 1; pass models[0] again when there is one model).  Both must be of one
+ * kind and take one input width, and each is validated on the host before any launch (MC_EINVAL otherwise).
+ * d_nrows[0] (device) rows, row_cap >= it.  d_ws: scratch of
  * mc_classify_workspace_bytes(row_cap) bytes (index list of the call rows, so the kernels run with every lane busy).
  */
 int64_t mc_classify_workspace_bytes(int64_t row_cap);

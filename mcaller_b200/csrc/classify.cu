@@ -580,15 +580,21 @@ extern "C" int mc_classify(mc_call *d_calls, const uint64_t *d_nrows, int64_t n_
     cudaStream_t st = (cudaStream_t)stream;
     const unsigned long long *dn = reinterpret_cast<const unsigned long long *>(d_nrows);
     const mc_model &m0 = models[0], &m1 = models[1];
-    MC_REQUIRE(m0.n_in >= 1 && m0.n_in <= MC_MAXK + 1, "model input width out of range");
+    // one kernel serves both models, so they must be of one kind; each is validated on its own
+    MC_REQUIRE(m0.kind == m1.kind, "models 0 ('MH') and 1 ('MG') are of different kinds");
+    MC_REQUIRE(m0.n_in >= 1 && m0.n_in <= MC_MAXK + 1, "model 0 ('MH') input width out of range");
+    MC_REQUIRE(m1.n_in == m0.n_in, "models 0 ('MH') and 1 ('MG') take different input widths");
     switch (m0.kind) {
         case MC_MLP: {
-            MC_REQUIRE(m0.n_layers >= 1 && m0.n_layers < 8, "MLP depth out of range");
-            for (int l = 0; l <= m0.n_layers; ++l) MC_REQUIRE(m0.sizes[l] >= 1 && m0.sizes[l] <= MAX_WIDTH, "MLP layer too wide");
-            MC_REQUIRE(m0.sizes[m0.n_layers] == 1, "MLP must have one logistic output");
+            for (const mc_model *m : {&m0, &m1}) {
+                MC_REQUIRE(m->n_layers >= 1 && m->n_layers < 8, "MLP depth out of range");
+                MC_REQUIRE(m->sizes[0] == m->n_in, "MLP input layer does not match its input width");
+                for (int l = 0; l <= m->n_layers; ++l) MC_REQUIRE(m->sizes[l] >= 1 && m->sizes[l] <= MAX_WIDTH, "MLP layer too wide");
+                MC_REQUIRE(m->sizes[m->n_layers] == 1, "MLP must have one logistic output");
+            }
             int width = 8;
             for (int l = 0; l <= m0.n_layers; ++l) width = m0.sizes[l] > width ? m0.sizes[l] : width;
-            for (int l = 0; l <= m1.n_layers && m1.kind == MC_MLP; ++l) width = m1.sizes[l] > width ? m1.sizes[l] : width;
+            for (int l = 0; l <= m1.n_layers; ++l) width = m1.sizes[l] > width ? m1.sizes[l] : width;
             width = (width + 3) & ~3;
             auto count = [](const mc_model &m, int &nw, int &nb) {
                 nw = nb = 0;
@@ -611,7 +617,7 @@ extern "C" int mc_classify(mc_call *d_calls, const uint64_t *d_nrows, int64_t n_
                 return m.kind == MC_MLP && m.n_layers == 2 && m.sizes[0] <= MLP_MAX_IN && m.sizes[2] == 1;
             };
             const size_t weight_bytes = sizeof(double) * (size_t)(nw0 + nb0 + nw1 + nb1);
-            if (one_hidden(m0) && (alias || m1.kind != MC_MLP || one_hidden(m1)) && weight_bytes <= 100 * 1024) {
+            if (one_hidden(m0) && (alias || one_hidden(m1)) && weight_bytes <= 100 * 1024) {
                 int64_t b2 = (n_calls + WARPS * 8 - 1) / (WARPS * 8);
                 if (b2 > (int64_t)sms * 8) b2 = (int64_t)sms * 8;
                 // index list of the MC_CALL rows first: [count (u64, 256-byte slot)][row indices u32]

@@ -394,7 +394,10 @@ k_windows(const mc_record *__restrict__ rec, int64_t rec_cap, const unsigned lon
                     const int clen = __ldg(R.d_len + last_cid);
                     uint8_t nextb = 0;
                     if (mpos - k + 1 < 0 || mpos + k > clen) err |= MC_CE_CONTEXT;
-                    else if (!last_rev) {
+                    else if (k < 2) {
+                        // the key context[k-1:k+1] of a one-letter context has one letter: KeyError in base_models
+                        // (nextb stays 0, which the check below flags as MC_CE_MODELKEY)
+                    } else if (!last_rev) {
                         const int64_t gn = g + 1;
                         nextb = ((__ldg(R.d_site_fwd + (gn >> 5)) >> (gn & 31)) & 1u) ? 'M' : __ldg(R.d_bases + gn);
                     } else {

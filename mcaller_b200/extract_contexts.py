@@ -278,9 +278,7 @@ class RangeRun(object):
         if not train:
             model = _models.load_model_file(modelfile)
             e0, e1, two = _models.select_models(model, base)
-            dm = _models.DeviceModels(e0, e1)
-            if dm.n_in != k + 1:
-                raise ValueError("model expects %d inputs but -n %d gives %d" % (dm.n_in, k, k + 1))
+            dm = _models.DeviceModels(e0, e1, n_in=k + 1)     # both models' widths are checked before any export
         # read2qual: the reference's dict, or a read_qual.DeviceQualityTable built on the GPU from the FASTQ
         qt = read2qual if isinstance(read2qual, _rq.DeviceQualityTable) else _rq.build_quality_table(read2qual)
         if isinstance(qt, _rq.DeviceQualityTable) and qt.table.device.index != self.device_index:

@@ -43,10 +43,36 @@ def select_models(model, base):
     raise KeyError("model dict has neither MG/MH (base A) nor 'general'")
 
 
-class DeviceModels(object):
-    """Two mc_model structs (index 0 = 'MH'/'general', 1 = 'MG') backed by device tensors."""
+def input_width(est):
+    """Number of features a supported estimator takes (read from its fitted parameters, so older pickles without
+    n_features_in_ work too)."""
+    tn = type(est).__name__
+    if tn == "MLPClassifier":
+        return int(est.coefs_[0].shape[0])
+    if tn == "LogisticRegression":
+        return int(est.coef_.shape[1])
+    if tn == "GaussianNB":
+        return int(est.theta_.shape[1])
+    if tn == "RandomForestClassifier":
+        return int(est.n_features_in_)
+    raise TypeError("unsupported estimator type %s (supported: MLPClassifier, RandomForestClassifier, LogisticRegression, GaussianNB)" % tn)
 
-    def __init__(self, est0, est1=None, device="cuda"):
+
+class DeviceModels(object):
+    """Two mc_model structs (index 0 = 'MH'/'general', 1 = 'MG') backed by device tensors.  Both must be of one estimator
+    type: mc_classify runs one kernel for all rows (the reference would apply each key's estimator on its own; mCaller's
+    own training never writes a mixed dict).  `n_in`: the input width both must have (k + 1); checked, like the types,
+    before anything is copied to the device."""
+
+    def __init__(self, est0, est1=None, device="cuda", n_in=None):
+        if est1 is not None and type(est0).__name__ != type(est1).__name__:
+            raise TypeError("model dict mixes estimator types: 'MH' is %s, 'MG' is %s (both keys must have one type)"
+                            % (type(est0).__name__, type(est1).__name__))
+        if n_in is not None:
+            named = (("model 'MH'", est0), ("model 'MG'", est1)) if est1 is not None else (("model", est0),)
+            for what, est in named:
+                if input_width(est) != n_in:
+                    raise ValueError("%s expects %d inputs but -n %d gives %d" % (what, input_width(est), n_in - 1, n_in))
         self.device = torch.device(device)
         self._keep = []
         arr = (Model * 2)()

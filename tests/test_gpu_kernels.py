@@ -162,42 +162,271 @@ def test_device_generator_matches_numpy_generator(cuda_lib):
     assert d2[:n2].cpu().numpy().tobytes() == host_bytes[int(o[3]):int(o[8])]
 
 
-@pytest.mark.parametrize("kind,tol", [("RF", 1e-12), ("LR", 1e-12), ("NBC", 1e-10), ("NN", 1e-12)])
-def test_classifiers_match_sklearn(kind, tol, cuda_lib, oracle):
-    """mc_classify on synthetic feature rows vs scikit-learn predict_proba (float64 on both sides)."""
-    import torch
-    from mcaller_b200 import _lib, models
-    from test_oracle_numerics import _X, _fit_alt
-    if kind == "NN":
+def _Xw(n, d, seed):
+    """n feature rows of width d: column means around 0, then a read quality (as test_oracle_numerics._X for d = 7)."""
+    rng = np.random.default_rng(seed)
+    X = rng.normal(0, 3, (n, d))
+    X[:, d - 1] = rng.uniform(3, 20, n)
+    return X
+
+
+def _y(X, seed):
+    rng = np.random.default_rng(seed)
+    z = X[:, 0] - 0.5 * X[:, min(1, X.shape[1] - 1)] + rng.normal(0, 1.5, len(X))
+    return np.where(z > np.median(z), "m6A", "A")
+
+
+def _mlp(n_in, hidden, act, seed):
+    """A seeded MLPClassifier of the given shape; a few iterations: the shape matters, not the fit."""
+    import warnings
+    from sklearn.neural_network import MLPClassifier
+    X = _Xw(400, n_in, 50 + seed)
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        return MLPClassifier(hidden_layer_sizes=hidden, activation=act, max_iter=4, random_state=seed).fit(X, _y(X, seed))
+
+
+def _rf(seed, n=3000, d=7, **kw):
+    from sklearn.ensemble import RandomForestClassifier
+    X = _Xw(n, d, 70 + seed)
+    return RandomForestClassifier(random_state=seed, **kw).fit(X, _y(X, seed))
+
+
+def _rf_nodes(leaves):
+    """One tree grown to exactly `leaves` leaves (2 * leaves - 1 nodes) on label noise."""
+    from sklearn.ensemble import RandomForestClassifier
+    rng = np.random.default_rng(leaves)
+    X = rng.normal(size=(4 * leaves, 7))
+    rf = RandomForestClassifier(n_estimators=1, bootstrap=False, max_leaf_nodes=leaves, random_state=0).fit(X, rng.integers(0, 2, len(X)))
+    assert rf.estimators_[0].tree_.node_count == 2 * leaves - 1
+    return rf
+
+
+def _mlp_branch(est0, est1, alias=False):
+    """Which MLP kernel mc_classify launches (the dispatch rule of classify.cu, restated): '1hidden' (k_mlp_1hidden),
+    'staged' (k_mlp<true>) or 'global' (k_mlp<false>)."""
+    def sizes(e):
+        return [e.coefs_[0].shape[0]] + [c.shape[1] for c in e.coefs_]
+
+    def params(e):
+        s = sizes(e)
+        return sum(s[i] * s[i + 1] + s[i + 1] for i in range(len(s) - 1))
+
+    def one_hidden(e):
+        return len(e.coefs_) == 2 and sizes(e)[0] <= 9
+
+    width = max([8] + sizes(est0) + sizes(est1))
+    width = (width + 3) & ~3
+    weight_bytes = 8 * (params(est0) + (0 if alias else params(est1)))
+    if one_hidden(est0) and (alias or one_hidden(est1)) and weight_bytes <= 100 * 1024:
+        return "1hidden"
+    if 8 * 2 * width * 8 + weight_bytes <= 100 * 1024:
+        return "staged"
+    return "global"
+
+
+def _classifier_case(name):
+    """(est0 ('MH'), est1 ('MG'), input width, alias) of a classifier-matrix case."""
+    from mcaller_b200 import models
+    from test_oracle_numerics import _fit_alt
+    from sklearn.linear_model import LogisticRegression
+    from sklearn.naive_bayes import GaussianNB
+    if name == "NN":
         m = models.load_model_file(os.path.join(gc.GOLD, "models", gc.R95))
-        est0, est1 = m["MH"], m["MG"]
-    else:
-        est0 = est1 = _fit_alt(kind)
-    dm = models.DeviceModels(est0, est1)
-    X = _X(777, 13)
-    calls = np.zeros(len(X), dtype=_lib.CALL_DTYPE)
-    calls["feat"][:, :7] = X
-    calls["model_sel"] = np.arange(len(X)) % 2
-    calls["kind"][::50] = 1                       # non-call rows must be left untouched
-    # the row count lives on the device; the capacity only sizes the launch: the last 20 rows lie beyond the count
-    n_live = len(X) - 20
+        return m["MH"], m["MG"], 7, False
+    if name in ("RF", "LR", "NBC"):
+        e = _fit_alt(name)
+        return e, e, 7, False
+    f = name.split(":")
+    if f[0] == "1h":                               # 1h:<n_in>:<H>:<act>
+        n_in, H, act = int(f[1]), int(f[2]), f[3]
+        return _mlp(n_in, (H,), act, 1), _mlp(n_in, (H,), act, 2), n_in, False
+    if f[0] == "1h_alias":                         # one estimator for both keys, given once (model 1 aliases model 0)
+        e = _mlp(7, (100,), "tanh", 3)
+        return e, e, 7, True
+    if f[0] == "1h_same":                          # one estimator for both keys, exported twice
+        e = _mlp(7, (100,), "tanh", 3)
+        return e, e, 7, False
+    if name == "staged_64_32_relu":
+        return _mlp(7, (64, 32), "relu", 4), _mlp(7, (64, 32), "relu", 5), 7, False
+    if name == "staged_16_7_3_logistic":
+        return _mlp(7, (16, 7, 3), "logistic", 6), _mlp(7, (16, 7, 3), "logistic", 7), 7, False
+    if name == "staged_1h_with_2h":
+        return _mlp(7, (100,), "tanh", 8), _mlp(7, (40, 20), "tanh", 9), 7, False
+    if name.startswith("global_300_200_"):
+        act = name.rsplit("_", 1)[1]
+        return _mlp(7, (300, 200), act, 10), _mlp(7, (300, 200), act, 11), 7, False
+    if name == "RF_leaf":                          # every tree is a single leaf
+        e = _rf(1, n=200, n_estimators=4, min_samples_split=1000)
+        return e, e, 7, False
+    if name == "RF_sizes":                         # forests of different tree counts and node counts per key
+        return _rf(2, n_estimators=3, max_depth=4), _rf(3, n_estimators=7, max_depth=14), 7, False
+    if name == "RF_wide":
+        return _rf(4, d=9, n_estimators=5, max_depth=10), _rf(5, d=9, n_estimators=2), 9, False
+    if name == "RF_7313_nodes":                    # largest tree just under the shared-memory staging limit (7 314 nodes)
+        return _rf_nodes(3657), _rf_nodes(3657), 7, False
+    if name == "LR_wide":
+        X = _Xw(500, 3, 1)
+        return LogisticRegression().fit(X, _y(X, 1)), LogisticRegression(C=0.1).fit(X, _y(X, 2)), 3, False
+    if name == "NBC_tiny_smoothing":
+        X = _Xw(500, 9, 2)
+        return GaussianNB(var_smoothing=1e-15).fit(X, _y(X, 3)), GaussianNB().fit(X, _y(X, 4)), 9, False
+    raise KeyError(name)
+
+
+_MLP_1H = ["1h:%d:%d:%s" % (n_in, H, act) for n_in in (1, 5, 9) for H in (1, 3, 17, 100, 129, 512)
+           for act in ("identity", "logistic", "tanh", "relu") if act == "tanh" or H in (3, 129)]
+_MLP_OTHER = ["1h_alias", "1h_same", "staged_64_32_relu", "staged_16_7_3_logistic", "staged_1h_with_2h", "global_300_200_identity",
+              "global_300_200_relu"]
+_OTHER = ["RF_leaf", "RF_sizes", "RF_wide", "RF_7313_nodes", "LR_wide", "NBC_tiny_smoothing"]
+_TOL = {"NBC": 1e-10}
+_CLASSIFIER_CASES = ([pytest.param(k, t, None, id="%s-%s" % (k, t)) for k, t in [("RF", 1e-12), ("LR", 1e-12), ("NBC", 1e-10), ("NN", 1e-12)]]
+                     + [pytest.param(k, _TOL.get(k[:3], 1e-12), None, id=k) for k in _MLP_1H + _MLP_OTHER + _OTHER]
+                     + [pytest.param(k, _TOL.get(k, 1e-12), n, id="%s-rows%d" % (k, n))
+                        for k in ("NN", "staged_16_7_3_logistic", "global_300_200_relu", "RF", "LR", "NBC") for n in (0, 1, 33, 200000)])
+
+
+def test_classifier_matrix_reaches_every_mlp_kernel():
+    """The parametrization of test_classifiers_match_sklearn reaches each of the three MLP kernels, so a later change to
+    the dispatch rule cannot silently drop one from the tests."""
+    seen = {}
+    for name in _MLP_1H + _MLP_OTHER + ["NN"]:
+        e0, e1, _, alias = _classifier_case(name)
+        seen.setdefault(_mlp_branch(e0, e1, alias), []).append(name)
+    assert set(seen) == {"1hidden", "staged", "global"}
+    assert seen["staged"] == ["staged_64_32_relu", "staged_16_7_3_logistic", "staged_1h_with_2h"]
+    assert seen["global"] == ["global_300_200_identity", "global_300_200_relu"]
+
+
+def _run_classify(cuda_lib, model_array, calls, n_live):
+    import torch
+    from mcaller_b200 import _lib
     d = torch.from_numpy(calls.view(np.uint8).reshape(-1).copy()).cuda()
     d_n = torch.tensor([n_live], dtype=torch.int64, device="cuda")
-    d_ws = torch.zeros(int(cuda_lib.mc_classify_workspace_bytes(len(X))), dtype=torch.uint8, device="cuda")
-    _lib.check(cuda_lib.mc_classify(C.c_void_p(d.data_ptr()), C.c_void_p(d_n.data_ptr()), len(X), dm.array, C.c_void_p(d_ws.data_ptr()),
-                                    C.c_void_p(torch.cuda.current_stream().cuda_stream)))
-    out = d.cpu().numpy().view(_lib.CALL_DTYPE)
-    assert np.all(out["prob"][n_live:] == 0)
-    calls["kind"][n_live:] = 1
+    d_ws = torch.zeros(int(cuda_lib.mc_classify_workspace_bytes(len(calls))), dtype=torch.uint8, device="cuda")
+    rc = cuda_lib.mc_classify(C.c_void_p(d.data_ptr()), C.c_void_p(d_n.data_ptr()), len(calls), model_array, C.c_void_p(d_ws.data_ptr()),
+                              C.c_void_p(torch.cuda.current_stream().cuda_stream))
+    return rc, d.cpu().numpy().view(_lib.CALL_DTYPE)
+
+
+@pytest.mark.parametrize("kind,tol,rows", _CLASSIFIER_CASES)
+def test_classifiers_match_sklearn(kind, tol, rows, cuda_lib, oracle):
+    """mc_classify on synthetic feature rows vs scikit-learn predict_proba and the oracle's restatement (float64 on all
+    sides): every MLP kernel (the shipped shape, other input widths, hidden widths and activations, deeper and wider
+    nets), RF at its float32 split edges, single-leaf trees, forests of different sizes and the largest tree that fits the
+    shared-memory staging, LR and GaussianNB where p saturates to exactly 0 and 1.  Rows of another kind (every 50th),
+    rows beyond the device-side count and feature slots beyond the model's width (NaN here) must not be touched or read."""
     import warnings
+    from mcaller_b200 import _lib, models
+    est0, est1, n_in, alias = _classifier_case(kind)
+    dm = models.DeviceModels(est0, est1, n_in=n_in)
+    if alias:
+        dm.array[1] = dm.array[0]                 # model 1 is model 0: its weights are staged once
+        assert _mlp_branch(est0, est1, alias=True) == "1hidden"
+    n_live = 777 - 20 if rows is None else rows
+    X = _Xw(n_live + 20, n_in, 13)
+    sel = np.arange(len(X)) % 2
+    special = []                                  # (model selector, feature row) placed from row 1 on
+    if kind.startswith("RF"):
+        # features exactly at float32(threshold), one float32 ulp either side, and the float64 neighbours of the threshold
+        # (which may round to float32 on either side of it), each evaluated by the forest the threshold belongs to
+        for m, e in enumerate((est0, est1)):
+            tr = e.estimators_[0].tree_
+            for f, t in [(int(f), float(t)) for f, t in zip(tr.feature, tr.threshold) if f >= 0][:30]:
+                t32 = np.float32(t)
+                for v in (t32, np.nextafter(t32, np.float32(-np.inf)), np.nextafter(t32, np.float32(np.inf)), t, np.nextafter(t, -np.inf),
+                          np.nextafter(t, np.inf)):
+                    r = X[(len(special) + 1) % len(X)].copy()
+                    r[f] = float(v)
+                    special.append((m, r))
+    if kind.startswith(("LR", "NBC")):
+        # far out along each axis and the diagonal, both signs: p saturates to exactly 0 and exactly 1
+        for m in (0, 1):
+            for j in range(n_in + 1):
+                for sgn in (-1e3, 1e3):
+                    r = np.full(n_in, sgn) if j == n_in else np.zeros(n_in)
+                    if j < n_in:
+                        r[j] = sgn
+                    special.append((m, r))
+    all_special = len(special) < n_live       # room for every special row among the live ones (row 0 stays plain)
+    special = special[:max(0, n_live - 1)]
+    for r, (m, row) in enumerate(special):
+        X[r + 1], sel[r + 1] = row, m
+    calls = np.zeros(len(X), dtype=_lib.CALL_DTYPE)
+    calls["feat"][:, :n_in] = X
+    calls["feat"][:, n_in:] = np.nan
+    calls["model_sel"] = sel
+    calls["kind"][::50] = 1                       # non-call rows must be left untouched
+    # the row count lives on the device; the capacity only sizes the launch: the last 20 rows lie beyond the count
+    rc, out = _run_classify(cuda_lib, dm.array, calls, n_live)
+    _lib.check(rc)
+    assert np.all(out["prob"][n_live:] == 0) and np.all(out["label"][n_live:] == 0)
+    calls["kind"][n_live:] = 1
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         w0, w1 = est0.predict_proba(X)[:, 1], est1.predict_proba(X)[:, 1]
-    want = np.where(np.arange(len(X)) % 2 == 1, w1, w0)
+    want = np.where(sel == 1, w1, w0)
     live = calls["kind"] == 0
-    assert np.max(np.abs(out["prob"][live] - want[live])) < tol
+    assert np.max(np.abs(out["prob"][live] - want[live]), initial=0.0) < tol
     assert np.array_equal(out["label"][live], (want[live] >= 0.5).astype(np.uint8))
-    assert np.all(out["prob"][~live] == 0)
+    assert np.all(out["prob"][~live] == 0) and np.all(out["label"][~live] == 0)
+    if kind.startswith(("LR", "NBC")) and all_special:
+        assert {0.0, 1.0} <= set(want[live].tolist())
+    # the oracle's restatement of predict_proba, on all rows (a fixed sample of them for the largest count)
+    idx = np.flatnonzero(live)
+    if len(idx) > 3000:
+        idx = np.concatenate([idx[:1000], np.random.default_rng(0).choice(idx[1000:], 1000, replace=False)])
+    for m, est in ((0, est0), (1, est1)):
+        j = idx[sel[idx] == m]
+        if len(j):
+            assert np.max(np.abs(out["prob"][j] - oracle.predict(est, X[j]))) < tol
+
+
+def test_rf_tree_over_the_shared_memory_limit_is_refused(cuda_lib):
+    """A tree of 7 315 nodes does not fit the 200 KB shared-memory staging of k_rf: mc_classify refuses it on the host
+    (MC_EINVAL, McallerCudaError) and launches nothing."""
+    from mcaller_b200 import _lib, models
+    e = _rf_nodes(3658)
+    dm = models.DeviceModels(e, e, n_in=7)
+    calls = np.zeros(64, dtype=_lib.CALL_DTYPE)
+    calls["feat"][:, :7] = _Xw(64, 7, 1)
+    rc, out = _run_classify(cuda_lib, dm.array, calls, 64)
+    assert rc == -1                                # MC_EINVAL
+    with pytest.raises(_lib.McallerCudaError, match="RF tree too large"):
+        _lib.check(rc)
+    assert np.all(out["prob"] == 0) and np.all(out["label"] == 0)
+
+
+def _kind_est(kind):
+    from test_oracle_numerics import _fit_alt
+    if kind == "MLP":
+        return _mlp(7, (10,), "tanh", 1)
+    if kind == "RF":
+        return _rf(1, n=300, n_estimators=2, max_depth=3)
+    return _fit_alt(kind)
+
+
+_KINDS = ["MLP", "RF", "LR", "NBC"]
+
+
+@pytest.mark.parametrize("k0,k1", [(a, b) for a in _KINDS for b in _KINDS if a != b])
+def test_mixed_estimator_types_are_refused_on_the_host(k0, k1, cuda_lib):
+    """One classifier kernel serves both keys, so a dict whose 'MH' and 'MG' estimators differ in type is refused:
+    DeviceModels raises TypeError naming both before exporting anything, and mc_classify given such a pair (built by
+    hand) returns MC_EINVAL.  The device-side row count is 0, so no kernel could touch a row even without the check."""
+    from mcaller_b200 import _lib, models
+    e0, e1 = _kind_est(k0), _kind_est(k1)
+    with pytest.raises(TypeError, match="'MH' is %s, 'MG' is %s" % (type(e0).__name__, type(e1).__name__)):
+        models.DeviceModels(e0, e1)
+    d0, d1 = models.DeviceModels(e0), models.DeviceModels(e1)
+    arr = (_lib.Model * 2)()
+    arr[0], arr[1] = d0.array[0], d1.array[0]
+    calls = np.zeros(64, dtype=_lib.CALL_DTYPE)
+    calls["model_sel"] = np.arange(64) % 2
+    rc, out = _run_classify(cuda_lib, arr, calls, 0)
+    assert rc == -1                                # MC_EINVAL
+    assert "different kinds" in cuda_lib.mc_last_error().decode()
+    assert np.all(out["prob"] == 0)
 
 
 def test_histogram_matches_oracle_aggregation(tmp_path, cuda_lib, oracle):

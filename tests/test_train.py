@@ -129,19 +129,28 @@ def test_train_entry_points_declared_exported_and_bound():
 
 # ---- GPU ------------------------------------------------------------------------------------------------------------
 
-CASES = [(s, n) for s in (0, 1, 2) for n in (150, 20000, 20001)]
+# (seed, rows, input width): the shipped width 7, and 2 and 9 (-n 1 and -n 8), whose fits index every array by d
+CASES = [(s, n, 7) for s in (0, 1, 2) for n in (150, 20000, 20001)] + [(1, n, 2) for n in (150, 20001)] + [(2, n, 9) for n in (150, 20001)]
 
 
 @pytest.fixture(scope="module")
 def fits_vs_sklearn(cuda_lib):
-    """All cases as jobs of one call (rows 0..n of one matrix), plus a noisy 150-row set that runs to max_iter."""
+    """Per case (CASES, then a noisy 150-row set of width 7 that runs to max_iter): (x, y, rows, seed, fit result).  The
+    cases of one width are jobs of one call (rows 0..n of one matrix): fit_mlp_jobs takes one matrix."""
     from mcaller_b200 import train as tr
-    x, y = _blobs(20001, 7)
-    xm, ym = _blobs(150, 8, noise=3.0)
-    xa, ya = np.concatenate([x, xm]), np.concatenate([y, ym])
-    jobs = [(np.arange(n), s) for s, n in CASES] + [(20001 + np.arange(150), 3)]
-    res = tr.fit_mlp_jobs(xa, ya, jobs)
-    return xa, ya, jobs, res
+    out = {}
+    for d in sorted({c[2] for c in CASES}):
+        x, y = _blobs(20001, 7, d=d)
+        idx = [i for i, c in enumerate(CASES) if c[2] == d]
+        jobs = [(np.arange(CASES[i][1]), CASES[i][0]) for i in idx]
+        if d == 7:
+            xm, ym = _blobs(150, 8, noise=3.0)
+            x, y = np.concatenate([x, xm]), np.concatenate([y, ym])
+            idx.append(len(CASES))
+            jobs.append((20001 + np.arange(150), 3))
+        for i, job, r in zip(idx, jobs, tr.fit_mlp_jobs(x, y, jobs)):
+            out[i] = (x, y, job[0], job[1], r)
+    return out
 
 
 @pytest.mark.gpu
@@ -149,21 +158,21 @@ def fits_vs_sklearn(cuda_lib):
 def test_gpu_fit_matches_sklearn(case, fits_vs_sklearn):
     from sklearn.neural_network import MLPClassifier
     from mcaller_b200 import train as tr
-    xa, ya, jobs, res = fits_vs_sklearn
-    rows, seed = jobs[case]
+    xa, ya, rows, seed, res = fits_vs_sklearn[case]
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         ref = MLPClassifier(random_state=seed, **tr.SHIPPED_NN).fit(xa[rows], ya[rows])
-    params, n_iter, curve, best, noimp = res[case]
+    params, n_iter, curve, best, noimp = res
     if case == len(CASES):
         assert ref.n_iter_ == tr.SHIPPED_NN["max_iter"]
     assert n_iter == ref.n_iter_
     assert np.allclose(curve, ref.loss_curve_, rtol=1e-10, atol=0)
     W0, W1, c0, c1 = params
+    assert W0.shape == (xa.shape[1], 100)
     assert np.max(np.abs(W0 - ref.coefs_[0])) < 1e-9 and np.max(np.abs(W1 - ref.coefs_[1])) < 1e-9
     assert np.max(np.abs(c0 - ref.intercepts_[0])) < 1e-9 and np.max(np.abs(c1 - ref.intercepts_[1])) < 1e-9
     est = tr.make_mlp(params, [0.0, 1.0], xa.shape[1], n_iter, curve, best, len(rows), seed, noimp)
-    held, _ = _blobs(500, 99)
+    held, _ = _blobs(500, 99, d=xa.shape[1])
     assert np.allclose(est.predict_proba(held), ref.predict_proba(held), rtol=1e-10, atol=0)
     assert est.best_loss_ == pytest.approx(ref.best_loss_, rel=1e-10) and est.t_ == ref.t_
 
