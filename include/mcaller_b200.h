@@ -132,7 +132,7 @@ enum { MC_CALL = 0, MC_TOO_MANY_SKIPS = 1, MC_MULTI_M = 2, MC_NONE = 3 /* empty 
 #define MC_CE_CONTEXT 1u   /* window within k of a contig end (reference: IndexError / sys.exit, :195, :224) */
 #define MC_CE_MODELKEY 2u  /* base after the target not in ACGTM (reference: KeyError -> sys.exit, :218-223) */
 #define MC_CE_BADNUM 4u    /* a fed line had an unsupported numeric field */
-#define MC_CE_COLUMN 8u    /* columns with more than 128 events outgrew the spill arena of mc_build_windows */
+#define MC_CE_COLUMN 8u    /* a column holds 65535 or more events: its count saturated, the mean is not computed */
 #define MC_CE_SPACING 16u  /* multi-M shift of 0 (reference: 'n diffs off' -> sys.exit, :257-266) */
 
 /* ---- classifier (host struct holding device pointers; layout mirrors sklearn's fitted attributes) ---- */
@@ -261,10 +261,12 @@ int mc_segment_quality(const uint8_t *d_text, const mc_record *d_rec, const uint
  * (after which the reference's state is closed and empty); one thread per unit, two passes (count, exclusive scan,
  * write) so rows come out in file order.  d_rec must come from mc_order_records (MC_RF_SEGKNOWN / MC_RF_NEWREAD set)
  * and d_seg_start from mc_segment_reads on the same records.  d_seg_count is scratch of seg_cap uint32.  d_ncalls[0]
- * receives the number of rows (all kinds); rows beyond call_cap are dropped and d_ncalls[1] is set.  Segments whose
- * quality is below qual_thresh are skipped entirely (:167).  d_ws: mc_workspace_bytes(rec_cap).  d_spill (spill_cap doubles)
- * holds the values of columns with more than 128 events while numpy's recursive halving is replayed on them (a stalled
- * read); a chunk that needs more than spill_cap flags the row with MC_CE_COLUMN.
+ * receives the number of rows (all kinds).  Segments whose quality is below qual_thresh are skipped entirely (:167).
+ * d_ws: mc_workspace_bytes(rec_cap).  d_spill (spill_cap doubles) holds the values of columns with more than 128 events
+ * while numpy's recursive halving is replayed on them (a stalled read).  d_ncalls[1] is 0 when every buffer sufficed;
+ * otherwise bit 0 says rows beyond call_cap were dropped and bits 1-63 hold the doubles the spill arena would have needed
+ * when that is more than spill_cap (the rows of such columns are then wrong).  Either way the rows must be discarded and
+ * the chunk built again with larger buffers (mc_chunk_guard aborts on a nonzero d_ncalls[1]).
  */
 int mc_build_windows(const mc_record *d_rec, const uint64_t *d_n_records, int64_t rec_cap, const uint32_t *d_seg_start,
                      const uint64_t *d_nseg, int64_t seg_cap, const double *d_seg_qual, const mc_refindex *ref, int skip_thresh,

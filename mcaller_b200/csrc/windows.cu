@@ -171,9 +171,10 @@ __device__ __noinline__ double col_sum_big(const ColSrc S, uint32_t src, uint32_
         return res;
     }
     // more than 128 events in one column (a stalled read): numpy halves recursively, which needs the values side by side
-    // -> gather them into the spill arena
+    // -> gather them into the spill arena.  The cursor counts the demand of every such column, so after an overflow
+    // k_check_cap knows how large an arena the rerun of the chunk needs; the row written meanwhile is discarded.
     const unsigned long long at = atomicAdd(spill.cursor, (unsigned long long)n);
-    if (at + (unsigned long long)n > spill.cap) { *err |= MC_CE_COLUMN; return 0.0; }
+    if (at + (unsigned long long)n > spill.cap) return 0.0;
     double *a = spill.buf + at;
     int t = 0;
     for (uint32_t j = f0; j < upto; ++j)
@@ -343,7 +344,8 @@ k_windows(const mc_record *__restrict__ rec, int64_t rec_cap, const unsigned lon
         if (n < 8) res = s_seq[src * WIN_THREADS];                 // numpy adds fewer than 8 values left to right: the running sum
         else {
             const ColSrc S{s_rec, s_diff, rec, g_tag, base};
-            res = col_sum_big(S, (uint32_t)src, b, upto, n, spill, &err);
+            // numpy adds the pairwise sum to the reduction's initial 0.0: a column of -0.0 values sums to 0.0
+            res = __dadd_rn(col_sum_big(S, (uint32_t)src, b, upto, n, spill, &err), 0.0);
         }
         return __ddiv_rn(res, (double)n);
     };
@@ -571,8 +573,12 @@ k_windows(const mc_record *__restrict__ rec, int64_t rec_cap, const unsigned lon
     }
 }
 
-__global__ void k_check_cap(const unsigned long long *d_ncalls, unsigned long long cap, unsigned long long *d_flag) {
-    if (d_ncalls[0] > cap) *d_flag = 1ull;
+// d_flag = d_ncalls[1]: bit 0 = more rows than call_cap, bits 1-63 = the doubles the spill arena would have needed when
+// that is more than spill_cap (0 otherwise); nonzero makes mc_chunk_guard abort the chunk
+__global__ void k_check_cap(const unsigned long long *d_ncalls, unsigned long long cap, const unsigned long long *spill_cursor,
+                            unsigned long long spill_cap, unsigned long long *d_flag) {
+    const unsigned long long need = *spill_cursor;
+    *d_flag = (d_ncalls[0] > cap ? 1ull : 0ull) | (need > spill_cap ? need << 1 : 0ull);
 }
 
 }  // namespace
@@ -630,8 +636,8 @@ extern "C" int mc_build_windows(const mc_record *d_rec, const uint64_t *d_n_reco
                                                                   first_ind, *ref, skip_thresh, qual_thresh, two_models, d_calls,
                                                                   (unsigned long long)call_cap, unit_cnt, nullptr, blk_off, tags, spill);
     MC_LAUNCH_CHECK();
-    k_check_cap<<<1, 1, 0, st>>>(reinterpret_cast<unsigned long long *>(d_ncalls), (unsigned long long)call_cap,
-                                 reinterpret_cast<unsigned long long *>(d_ncalls) + 1);
+    k_check_cap<<<1, 1, 0, st>>>(reinterpret_cast<unsigned long long *>(d_ncalls), (unsigned long long)call_cap, spill_cursor,
+                                 (unsigned long long)spill_cap, reinterpret_cast<unsigned long long *>(d_ncalls) + 1);
     MC_LAUNCH_CHECK();
     return MC_OK;
 }

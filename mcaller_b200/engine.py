@@ -25,7 +25,8 @@ S_STATS = 24                # 7 row statistics of mc_count_calls
 S_WORDS = 32
 # persistent device state (uint64 slots): global row index of the next chunk's slot 0, rows in the odd-row list
 P_ROW_BASE, P_N_ODD, P_POISON = 0, 1, 2
-SPILL_CAP = 1 << 22         # doubles: values of columns with more than 128 events (a stalled read) while numpy's halving is replayed
+SPILL_CAP = 1 << 22         # doubles: values of columns with more than 128 events (a stalled read) while numpy's halving is replayed;
+                            # the initial size of the arena, which a chunk that needs more grows (and runs again)
 ODD_CAP = 1 << 16           # rows whose closing contig differs from their window's (reference quirk Q4); merged on the host
 
 
@@ -90,7 +91,8 @@ class Engine(object):
             self.d_carry = torch.zeros(CARRY_BYTES, dtype=torch.uint8, device=self.device)
             self.d_carry_out = torch.zeros(CALL_DTYPE.itemsize, dtype=torch.uint8, device=self.device)
             self.d_odd = torch.zeros(ODD_CAP * CALL_DTYPE.itemsize, dtype=torch.uint8, device=self.device)
-            self.d_spill = torch.zeros(SPILL_CAP, dtype=torch.float64, device=self.device)
+            self.spill_cap = SPILL_CAP
+            self.d_spill = torch.zeros(self.spill_cap, dtype=torch.float64, device=self.device)
             self.h_small = np.zeros(S_WORDS, dtype=np.uint64)
             self.rec_per_byte = self.call_per_byte = self.seg_per_byte = 0.0     # largest demand per text byte seen so far
             self.launches = 0
@@ -234,7 +236,12 @@ class Engine(object):
             elif n_seg > seg_cap:
                 seg_cap = min(n_seg + 1024, rec_cap)
             else:
-                call_cap = n_calls + 1024
+                over = int(cnt[S_CALL_OVERFLOW])           # k_check_cap: bit 0 rows over call_cap, bits 1-63 spill demand
+                if over & 1:
+                    call_cap = n_calls + 1024
+                if over >> 1:
+                    self.spill_cap = int((over >> 1) * 1.25)
+                    self.d_spill = torch.empty(self.spill_cap, dtype=torch.float64, device=self.device)
         if attempts:
             self.d_persist[P_POISON] = 0              # the overflow was handled here: nothing is pending for overflowed()
         res.counters = {nm: int(cnt[i]) for i, nm in enumerate(_lib.COUNTER_NAMES)}
@@ -286,7 +293,7 @@ class Engine(object):
         check(L.mc_build_windows(V(rec_b.data_ptr()), self._status_ptr(S_NREC), rec_cap, V(seg_start.data_ptr()), self._status_ptr(S_NSEG),
                                  seg_cap, V(seg_qual.data_ptr()), self.ref.ref(), self.skip_thresh, self.qual_thresh, self.two_models,
                                  rows1, call_cap, V(seg_count.data_ptr()), self._status_ptr(S_NCALLS), V(ws.data_ptr()),
-                                 V(self.d_spill.data_ptr()), SPILL_CAP, st))
+                                 V(self.d_spill.data_ptr()), self.spill_cap, st))
         check(L.mc_chunk_guard(V(self.d_small.data_ptr()), rec_cap, self._status_ptr(S_NREC), rec_cap, self._status_ptr(S_NSEG), seg_cap,
                                self._status_ptr(S_NCALLS), call_cap, self._status_ptr(S_ABORT), self._persist_ptr(P_POISON), st))
         check(L.mc_carry_rows(V(calls.data_ptr()), self._status_ptr(S_NCALLS), V(rec_b.data_ptr()), self._status_ptr(S_NREC),

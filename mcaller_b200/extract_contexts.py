@@ -192,6 +192,9 @@ def raise_row_error(err, mpos):
         raise ReferenceAbort("base after target %d is not one of ACGTM (reference: KeyError -> sys.exit, :218-223)" % mpos)
     if err & 4:
         raise ValueError("unsupported numeric field in a line feeding the window at %d" % mpos)
+    if err & 8:
+        raise ValueError("a column of the window at %d holds 65535 or more events, the most the window builder counts per "
+                         "column (the reference has no such limit, DESIGN.md section 8)" % mpos)
     if err & 16:
         raise ReferenceAbort("n diffs off (multi-M spacing 0) at %d" % mpos)
 

@@ -121,7 +121,8 @@ static double np_pairwise(const double *a, int64_t n) {
     }
 }
 
-double orc_np_mean(const double *a, int64_t n) { return np_pairwise(a, n) / (double)n; }
+/* add.reduce adds the pairwise sum to its initial 0.0, so a sum of -0.0 values comes out as 0.0 */
+double orc_np_mean(const double *a, int64_t n) { return (np_pairwise(a, n) + 0.0) / (double)n; }
 
 /* np.round(x, 4): multiply, rint, divide (numpy/_core/src/multiarray/calculation.c PyArray_Round) */
 double orc_np_round(double x, int decimals) {

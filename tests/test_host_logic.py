@@ -312,3 +312,15 @@ def test_multigpu_run_reports_a_failed_rank(tmp_path):
     from mcaller_b200 import multigpu
     with pytest.raises(RuntimeError, match="rank [01] of 2 exited"):
         multigpu.run(dict(tsv=str(tmp_path / "missing.eventalign.tsv"), k=6), 2)
+
+
+def test_every_row_error_flag_raises():
+    """A row carrying any MC_CE_* flag must stop the writer and the training export; a column of 65 535 or more events
+    (MC_CE_COLUMN, the window builder's per-column count limit) raises ValueError naming the limit."""
+    from mcaller_b200 import _lib
+    for flag in (_lib.MC_CE_CONTEXT, _lib.MC_CE_MODELKEY, _lib.MC_CE_BADNUM, _lib.MC_CE_COLUMN, _lib.MC_CE_SPACING):
+        with pytest.raises((ec.ReferenceAbort, ValueError)):
+            ec.raise_row_error(flag, 1234)
+    with pytest.raises(ValueError, match=r"window at 1234 holds 65535 or more events"):
+        ec.raise_row_error(_lib.MC_CE_COLUMN, 1234)
+    ec.raise_row_error(0, 1234)

@@ -10,14 +10,25 @@ import pytest
 import golden_cases as gc
 
 
+def _bits(x):
+    return np.float64(x).view(np.uint64)
+
+
 def test_np_mean_order(oracle):
+    """orc_np_mean equals np.mean as bits (the sign of a zero included): every count numpy sums differently (left to right
+    below 8, 8 lanes and a tail up to 128, recursive halving above, counts past numpy's 8192-element buffer), and columns
+    of -0.0 values, which numpy's reduction turns into 0.0 by starting it from 0.0."""
     L = oracle.lib()
     rng = np.random.default_rng(1)
-    for n in list(range(1, 40)) + [64, 127, 128, 129, 200, 300, 1000]:
-        for _ in range(50):
+    for n in list(range(1, 40)) + [64, 127, 128, 129, 200, 300, 1000, 4097, 8193, 65534, 100000]:
+        for _ in range(50 if n <= 1000 else 3):
             a = np.round(rng.uniform(-20, 20, n), 4)
             got = L.orc_np_mean(a.ctypes.data_as(C.c_void_p), C.c_int64(n))
-            assert got == float(np.mean(list(a))), n
+            assert _bits(got) == _bits(np.mean(list(a))), n
+    for n in (1, 7, 8, 129):
+        a = np.full(n, -0.0)
+        got = L.orc_np_mean(a.ctypes.data_as(C.c_void_p), C.c_int64(n))
+        assert _bits(got) == _bits(np.mean(list(a))) == _bits(0.0), n
 
 
 def test_np_round4(oracle):
