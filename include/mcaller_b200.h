@@ -404,6 +404,49 @@ int mc_diffs_rows(const uint8_t *d_text, int64_t nbytes, const uint64_t *d_posse
 int mc_diffs_colstats(const uint8_t *d_text, const mc_diffs_row *d_rows, const uint32_t *d_order, int64_t n_rows,
                       const uint32_t *d_locus_off, int64_t n_loci, int ncols, double *d_vals, uint32_t *d_ncol,
                       double *d_stats, uint64_t *d_counters, void *stream);
+/* The statistics half of mc_diffs_colstats on values already in d_vals[n_rows][MC_MAXK + 1] / d_ncol[n_rows] (grouped by
+ * the CSR d_locus_off[n_loci + 1]): d_stats[n_loci][ncols][2] = np.mean(x), np.add.reduce((x - mean)**2). */
+int mc_colstats(const double *d_vals, const uint32_t *d_ncol, const uint32_t *d_locus_off, int64_t n_loci, int ncols, double *d_stats,
+                void *stream);
+
+/*
+ * Row log of the multi-GPU product path (mCaller --gpus N --bed --bed_vo / --bed_positions): the per-read lists of
+ * make_bed.py --vo (:96-97, :147-159) and -p (:115-127) kept from the device rows instead of re-read from `.diffs` text.
+ *
+ * mc_rowlog_append: appends one mc_row_entry per row that mc_hist_accumulate counts (MC_CALL, closed, no error flag) to
+ *   d_log, in no particular order; with n_feat > 0 the entry is followed by the row's first n_feat features (empty
+ *   columns as 0.0, as the `.diffs` text prints them), so entries are mc_rowlog_stride(n_feat) bytes apart.  row_index:
+ *   d_row_base[0] + i, the index mc_hist_accumulate feeds to the first-seen minimum (run it before that call, which advances
+ *   the base); d_row_base NULL: the row carries its index in pad1/pad2 (mc_carry_close's output row), and a row closed by
+ *   another contig's line is skipped there as mc_carry_close skips it.  Rows closed by another contig's line get site -1.
+ *   d_site_flags (may be NULL: every row): only rows of site slots with a nonzero flag are logged (rows with site -1 always
+ *   are).  d_nrows NULL: row_cap rows.  d_n_log[0] is advanced by the rows logged, and so is d_n_added[0] (may be NULL: a
+ *   per-chunk count the host reads with the chunk's status, to size the log for the next chunk); entries past log_cap
+ *   are not written (the caller sizes d_log from the row capacity and checks d_n_log[0] <= log_cap).  d_abort: see
+ *   mc_chunk_guard.
+ * mc_rowlog_group: orders the gathered log by locus, first-seen order, and by row index inside a locus (the file order of the
+ *   reference's per-locus lists).  Locus of an entry: d_locus_of_site[site] (-1: not reported), or for site -1 the locus of
+ *   its row index in d_odd_rows[n_odd] (ascending) / d_odd_locus.  d_depth[n_loci + 1] holds each locus's row count (last
+ *   entry 0); d_locus_off[n_loci + 1] receives their exclusive scan, n_rows its total.  Outputs in grouped order:
+ *   d_prob[n_rows], and when d_vals is not NULL the features d_vals[n_rows][MC_MAXK + 1] with d_ncol[n_rows] = n_feat (the
+ *   input of mc_colstats).  d_counters[2]: entries of no reported locus, entries beyond their locus's count.
+ *   d_ws: mc_rowlog_group_workspace_bytes(n_rows, n_loci).
+ */
+typedef struct mc_row_entry {
+    uint64_t row;              /* global row index (first-seen order) */
+    int32_t site;              /* site slot, -1 for a row closed by another contig's line */
+    uint32_t pad;
+    double prob;               /* P(methylated) as classified */
+} mc_row_entry;                /* 24 bytes, then n_feat doubles */
+int64_t mc_rowlog_stride(int32_t n_feat);
+int mc_rowlog_append(const mc_call *d_calls, const uint64_t *d_nrows, int64_t row_cap, const uint64_t *d_row_base,
+                     const uint8_t *d_site_flags, int64_t n_sites, int32_t n_feat, void *d_log, int64_t log_cap, uint64_t *d_n_log,
+                     uint64_t *d_n_added, const uint64_t *d_abort, void *stream);
+int64_t mc_rowlog_group_workspace_bytes(int64_t n_rows, int64_t n_loci);
+int mc_rowlog_group(const void *d_log, int64_t n_entries, int32_t n_feat, const int32_t *d_locus_of_site, int64_t n_sites,
+                    const uint64_t *d_odd_rows, const int32_t *d_odd_locus, int64_t n_odd, const uint32_t *d_depth, int64_t n_loci,
+                    int64_t n_rows, uint32_t *d_locus_off, double *d_prob, double *d_vals, uint32_t *d_ncol, void *d_ws,
+                    uint64_t *d_counters, void *stream);
 
 /*
  * Host-side writer (no device work): renders the MC_CALL rows of a chunk (host copy of the mc_call array; rows still
@@ -421,6 +464,9 @@ int64_t mc_format_rows(const mc_call *h_calls, int64_t n_calls, const uint8_t *h
                        const char *const *marked_rev, const int64_t *contig_len, int32_t n_contigs, int32_t k,
                        const char *base_label, const char *mod_label, int32_t with_prob, int32_t max_threads, char *out,
                        int64_t out_cap);
+/* The probability column of mc_format_rows (np.round(p, 2) as str) for each of h_prob[n], written back to back into out;
+ * h_offsets[n + 1] receives where each string starts.  Returns the bytes written or MC_ECAPACITY (32 * n always suffices). */
+int64_t mc_format_probs(const double *h_prob, int64_t n, int32_t max_threads, char *out, int64_t out_cap, int64_t *h_offsets);
 
 /*
  * FASTQ read-quality ingest (reference read_qual.py:6-19) on the device.  mc_fastq_index builds the byte offset of every

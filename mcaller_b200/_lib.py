@@ -77,6 +77,8 @@ assert QUAL_DTYPE.itemsize == 24
 DIFFS_ROW_DTYPE = np.dtype([("line_off", "<u8"), ("slot", "<u4"), ("values_off", "<u4"), ("values_len", "<u4"), ("prob_off", "<u4"),
                             ("prob_len", "<u4"), ("pad", "<u4")])
 assert DIFFS_ROW_DTYPE.itemsize == 32
+ROW_ENTRY_DTYPE = np.dtype([("row", "<u8"), ("site", "<i4"), ("pad", "<u4"), ("prob", "<f8")])    # mc_row_entry, then n_feat doubles
+assert ROW_ENTRY_DTYPE.itemsize == 24
 
 
 class McallerCudaError(RuntimeError):
@@ -151,6 +153,19 @@ _PROTOS = {
     "mc_mlp_train_epochs": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "mc_diffs_colstats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
+    # d_vals, d_ncol, d_locus_off, n_loci, ncols, d_stats, stream
+    "mc_colstats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
+    "mc_rowlog_stride": (C.c_int64, [C.c_int32]),
+    # d_calls, d_nrows, row_cap, d_row_base, d_site_flags, n_sites, n_feat, d_log, log_cap, d_n_log, d_n_added, d_abort, stream
+    "mc_rowlog_append": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mc_rowlog_group_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64]),
+    # d_log, n_entries, n_feat, d_locus_of_site, n_sites, d_odd_rows, d_odd_locus, n_odd, d_depth, n_loci, n_rows, d_locus_off, d_prob,
+    # d_vals, d_ncol, d_ws, d_counters, stream
+    "mc_rowlog_group": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                  C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    # h_prob, n, max_threads, out, out_cap, h_offsets
+    "mc_format_probs": (C.c_int64, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
 }
 
 # symbols every build must export (checked by the CPU test-suite against include/mcaller_b200.h)

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmcaller_b200.so")
-SOURCES = ["api.cu", "scan.cu", "records.cu", "windows.cu", "classify.cu", "synth.cu", "aggregate.cu", "fastq.cu", "format.cu", "train.cu"]
+SOURCES = ["api.cu", "scan.cu", "records.cu", "windows.cu", "classify.cu", "synth.cu", "aggregate.cu", "fastq.cu", "format.cu", "train.cu", "rowlog.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "-shared"]
 

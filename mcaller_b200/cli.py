@@ -10,7 +10,9 @@ like the reference (mCaller.py:63-68); range i is handled on GPU i mod n_gpus, o
 `--gpus N` (extension) runs N ranks at once, one process per GPU (mcaller_b200.multigpu): rows are written per rank and
 concatenated, the per-site histograms are all-reduced over NCCL, and with `--bed` rank 0 writes make_bed.py's BED / GFF
 straight from the combined histogram (`--bed_min_read_depth`, `--bed_mod_threshold`, `--bed_control`, `--bed_gff`,
-`--bed_ref` mirror make_bed.py's -d / -t / --control / --gff / --ref).
+`--bed_ref` mirror make_bed.py's -d / -t / --control / --gff / --ref).  `--bed_vo` and `--bed_positions FILE` mirror
+make_bed.py's per-read modes --vo and -p FILE: the ranks keep the rows of each locus on the device and rank 0 writes the
+probability lists and per-column t-tests from them, again without any `.diffs` text.
 """
 import os
 import sys
@@ -44,8 +46,14 @@ def mcaller_main(argv=None):
     p.add_argument("--bed_control", action="store_true")
     p.add_argument("--bed_gff", action="store_true")
     p.add_argument("--bed_ref", type=str)
+    p.add_argument("--bed_vo", action="store_true", help="with --gpus --bed: make_bed.py --vo (per-locus probability lists)")
+    p.add_argument("--bed_positions", type=str, help="with --gpus --bed: make_bed.py -p FILE (listed loci, per-column t-tests)")
     p.add_argument("--seed", type=int, default=0, help="random_state of the training's balancing, folds and fits")
     a = p.parse_args(argv)
+    if (a.bed_vo or a.bed_positions) and not (a.gpus and a.gpus > 0 and a.bed):
+        p.error("--bed_vo and --bed_positions need --gpus N --bed")
+    if a.bed_positions:
+        assert os.path.isfile(a.bed_positions), "positions file not found at " + a.bed_positions
     if a.base == "A":
         mod = "m6A"
     elif a.base == "C":
@@ -66,7 +74,8 @@ def mcaller_main(argv=None):
         print("%d GPUs" % a.gpus)
         multigpu.run(dict(tsv=a.tsv, reference=a.reference, fastq=a.fastq, modelfile=modelfile, k=k, skip=a.skip_thresh, qual=a.qual_thresh,
                           base=base, motif=a.motif, positions=a.positions, bed=a.bed, bed_depth=a.bed_min_read_depth,
-                          bed_thresh=a.bed_mod_threshold, bed_control=a.bed_control, bed_gff=a.bed_gff, bed_ref=a.bed_ref), a.gpus)
+                          bed_thresh=a.bed_mod_threshold, bed_control=a.bed_control, bed_gff=a.bed_gff, bed_ref=a.bed_ref,
+                          bed_vo=a.bed_vo, bed_positions=a.bed_positions), a.gpus)
         print("Finished extracting signals")
         return 0
     read2qual = read_qual.extract_read_quality_device(a.fastq)        # FASTQ scanned on the GPU (same mapping as read_qual.py)

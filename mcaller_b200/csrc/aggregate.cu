@@ -384,8 +384,16 @@ extern "C" int mc_diffs_colstats(const uint8_t *d_text, const mc_diffs_row *d_ro
     k_diffs_values<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(d_text, d_rows, d_order, n_rows, d_vals, d_ncol,
                                                                      reinterpret_cast<unsigned long long *>(d_counters));
     MC_LAUNCH_CHECK();
+    return mc_colstats(d_vals, d_ncol, d_locus_off, n_loci, ncols, d_stats, stream);
+}
+
+extern "C" int mc_colstats(const double *d_vals, const uint32_t *d_ncol, const uint32_t *d_locus_off, int64_t n_loci, int ncols,
+                           double *d_stats, void *stream) {
+    MC_REQUIRE(d_vals && d_ncol && d_locus_off && d_stats, "null pointer");
+    MC_REQUIRE(ncols >= 1 && ncols <= MC_MAXK + 1, "column count out of range");
+    if (n_loci <= 0) return MC_OK;
     const int64_t nt = n_loci * ncols;
-    k_diffs_colstats<<<(unsigned)((nt + 127) / 128), 128, 0, st>>>(d_vals, d_ncol, d_locus_off, n_loci, ncols, d_stats);
+    k_diffs_colstats<<<(unsigned)((nt + 127) / 128), 128, 0, (cudaStream_t)stream>>>(d_vals, d_ncol, d_locus_off, n_loci, ncols, d_stats);
     MC_LAUNCH_CHECK();
     return MC_OK;
 }

@@ -22,7 +22,8 @@ extern "C" int mc_read_u64(const uint64_t *d_src, int64_t n, uint64_t *h_dst, vo
 }
 
 // struct sizes, so bindings in other languages can verify their layout (0 record, 1 call, 2 refindex, 3 model,
-// 4 qual entry, 5 synth spec, 6 locus entry, 7 diffs row, 8 carry, 9 training job)
+// 4 qual entry, 5 synth spec, 6 locus entry, 7 diffs row, 8 carry, 9 training job,
+// 10 row-log entry)
 extern "C" int mc_sizeof(int what) {
     switch (what) {
         case 0: return (int)sizeof(mc_record);
@@ -35,6 +36,7 @@ extern "C" int mc_sizeof(int what) {
         case 7: return (int)sizeof(mc_diffs_row);
         case 8: return (int)sizeof(mc_carry);
         case 9: return (int)sizeof(mc_train_job);
+        case 10: return (int)sizeof(mc_row_entry);
         default: return -1;
     }
 }

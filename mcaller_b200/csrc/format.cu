@@ -65,6 +65,9 @@ void put_int(Out &o, long long v) {
     o.put(b, (size_t)(r.ptr - b));
 }
 
+// the probability column: np.round(p, 2) printed as str(np.float64)
+void put_prob(Out &o, double p) { put_repr(o, std::rint(p * 100.0) / 100.0); }
+
 char comp(char c) {
     switch (c) { case 'A': return 'T'; case 'C': return 'G'; case 'G': return 'C'; case 'T': return 'A'; case 'N': return 'N'; case 'M': return 'M'; }
     return 0;
@@ -137,7 +140,7 @@ int64_t format_range(const FormatArgs &A, int64_t lo, int64_t hi, std::string &d
             o.put('\t');
             o.put(c.prob >= 0.5 ? A.mod_label : A.base_label);
             o.put('\t');
-            put_repr(o, std::rint(c.prob * 100.0) / 100.0);
+            put_prob(o, c.prob);
         }
         o.put('\n');
         if (!o.ok) { err_row = i; err_flags = -3; return MC_ECAPACITY; }       // cannot happen: labels are short
@@ -202,5 +205,47 @@ extern "C" int64_t mc_format_rows(const mc_call *h_calls, int64_t n_calls, const
     if (total > out_cap) { mc_set_error("mc_format_rows: output buffer too small"); return MC_ECAPACITY; }
     char *p = out;
     for (auto &sp : parts) { memcpy(p, sp.data(), sp.size()); p += sp.size(); }
+    return total;
+}
+
+extern "C" int64_t mc_format_probs(const double *h_prob, int64_t n, int32_t max_threads, char *out, int64_t out_cap, int64_t *h_offsets) {
+    if ((n > 0 && (!h_prob || !out)) || !h_offsets || n < 0) {
+        mc_set_error("mc_format_probs: bad argument");
+        return MC_EINVAL;
+    }
+    // a string is at most 24 bytes ("-1.2345678901234567e-05"), so slices of the output fit 32 bytes per value
+    if (out_cap < 32 * n) { mc_set_error("mc_format_probs: output buffer too small"); return MC_ECAPACITY; }
+    unsigned hw = std::thread::hardware_concurrency();
+    if (hw == 0) hw = 1;
+    if (max_threads > 0 && (unsigned)max_threads < hw) hw = (unsigned)max_threads;
+    int nt = (int)((n + 65535) / 65536);                            // ~65k values per thread (~5 ms of rendering)
+    if (nt > (int)hw) nt = (int)hw;
+    if (nt < 1) nt = 1;
+    // thread t renders values [lo, hi) into out[32 lo, 32 hi) with offsets relative to its slice; then the slices are packed
+    std::vector<int64_t> used((size_t)nt, 0);
+    auto work = [&](int t) {
+        const int64_t lo = n * t / nt, hi = n * (t + 1) / nt;
+        Out o{out + 32 * lo, out + 32 * hi};
+        for (int64_t i = lo; i < hi; ++i) {
+            h_offsets[i] = (int64_t)(o.p - (out + 32 * lo));
+            put_prob(o, h_prob[i]);
+        }
+        used[(size_t)t] = (int64_t)(o.p - (out + 32 * lo));
+    };
+    if (nt == 1) work(0);
+    else {
+        std::vector<std::thread> th;
+        for (int t = 1; t < nt; ++t) th.emplace_back(work, t);
+        work(0);
+        for (auto &x : th) x.join();
+    }
+    int64_t total = 0;
+    for (int t = 0; t < nt; ++t) {
+        const int64_t lo = n * t / nt, hi = n * (t + 1) / nt;
+        if (total != 32 * lo) memmove(out + total, out + 32 * lo, (size_t)used[(size_t)t]);
+        for (int64_t i = lo; i < hi; ++i) h_offsets[i] += total;
+        total += used[(size_t)t];
+    }
+    h_offsets[n] = total;
     return total;
 }

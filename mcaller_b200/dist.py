@@ -3,9 +3,11 @@ collective.  The only exchanges are, once per byte range,
 (1) one all-gather of an int64 per rank -- the contig of the rank's first kept line: the window a rank leaves open at the
     end of its slice is closed by the first kept line of the next rank that has one (reference semantics of
     extract_contexts.py:179 across the byte-range split of mCaller.py:63-68); the result stays on the device and is
-    consumed there by mc_carry_close, and
+    consumed there by mc_carry_close,
 (2) the all-reduce of the per-site histograms: one SUM over the packed depth|meth counts, one MIN over the first-seen
-    row indices (NCCL over NVLink on the GPU box, gloo in the CPU tests)."""
+    row indices (NCCL over NVLink on the GPU box, gloo when several ranks share a GPU), and
+(3) only when a per-read summary is asked for (make_bed --vo / -p: `--bed_vo`, `--bed_positions`), the gather of every
+    rank's row log to rank 0: one all-gather of the entry counts, one gather of the entries."""
 import torch
 import torch.distributed as dist
 
@@ -61,3 +63,34 @@ def close_and_reduce(engine, rank, group=None, fetch=True):
     else:
         allreduce_histogram(engine.d_counts, engine.d_first, group)
     return row
+
+
+def gather_row_log(engine, rank, group=None, dst=0):
+    """Every rank's row log (Engine.enable_row_log) -> rank `dst`: one all-gather of the counts, one gather of the entries.
+    A gather moves equal sizes, so each rank sends max-count entries and `dst` receives them into one buffer of world x
+    max-count entries, which the padding is then squeezed out of: with ranks of very different log sizes that buffer is
+    up to world times the entries kept.  Returns (uint8 device tensor of the entries in rank order, their count) on `dst`,
+    (None, 0) elsewhere.  Under gloo both steps are staged through host memory."""
+    host = dist.get_backend(group) == "gloo"
+    world = dist.get_world_size(group)
+    d_log, n = engine.row_log()
+    stride = engine.log_stride
+    cnt = torch.tensor([n], dtype=torch.int64, device="cpu" if host else engine.device)
+    counts = torch.empty(world, dtype=torch.int64, device=cnt.device)
+    dist.all_gather_into_tensor(counts, cnt, group=group)
+    counts = counts.tolist()
+    width = max(max(counts), 1) * stride
+    dev = "cpu" if host else engine.device
+    send = torch.zeros(width, dtype=torch.uint8, device=dev)
+    send[:n * stride].copy_(d_log)
+    recv = torch.empty(world, width, dtype=torch.uint8, device=dev) if rank == dst else None
+    dist.gather(send, list(recv.unbind(0)) if recv is not None else None, dst=dst, group=group)
+    if rank != dst:
+        return None, 0
+    total = int(sum(counts))
+    out = torch.empty(total * stride, dtype=torch.uint8, device=engine.device)
+    o = 0
+    for r, c in enumerate(counts):
+        out[o:o + c * stride].copy_(recv[r, :c * stride])
+        o += c * stride
+    return out, total

@@ -21,10 +21,12 @@ C_LINES, C_KEPT, C_RECORDS, C_SHORT, C_UNKNOWN, C_NNN, C_BADPOS, C_LONGLINE, C_O
 
 # layout of the per-chunk status block (uint64 slots): 0..15 the counters of mc_scan, then
 S_NSEG, S_MISSING_QUAL, S_NCALLS, S_CALL_OVERFLOW, S_ABORT, S_NREC, S_NROWS = 16, 17, 18, 19, 20, 21, 22
+S_NLOG = 23                 # entries mc_rowlog_append added in this chunk (row log enabled only)
 S_STATS = 24                # 7 row statistics of mc_count_calls
 S_WORDS = 32
-# persistent device state (uint64 slots): global row index of the next chunk's slot 0, rows in the odd-row list
-P_ROW_BASE, P_N_ODD, P_POISON = 0, 1, 2
+# persistent device state (uint64 slots): global row index of the next chunk's slot 0, rows in the odd-row list, the sticky
+# overflow flag, entries in the row log
+P_ROW_BASE, P_N_ODD, P_POISON, P_N_LOG = 0, 1, 2, 3
 SPILL_CAP = 1 << 22         # doubles: values of columns with more than 128 events (a stalled read) while numpy's halving is replayed;
                             # the initial size of the arena, which a chunk that needs more grows (and runs again)
 ODD_CAP = 1 << 16           # rows whose closing contig differs from their window's (reference quirk Q4); merged on the host
@@ -98,6 +100,7 @@ class Engine(object):
             self.launches = 0
             self.redone = 0                   # chunks run a second time because a buffer was too small
             self.scan_events = None           # set to [] to collect (start, end) CUDA events around the scan kernel
+            self.d_log = None                 # row log (enable_row_log): off unless a per-read summary is asked for
             self.reset_stream_state()
 
     # ---- buffers -----------------------------------------------------------------------------------------------
@@ -147,7 +150,58 @@ class Engine(object):
     def reset_histogram(self, row_base=0):
         self.d_counts.zero_()
         self.d_first.fill_(2 ** 63 - 1)
+        if self.d_log is not None:
+            self.d_persist[P_N_LOG] = 0
+            self.log_bound = 0
         self.reset_stream_state(row_base)
+
+    # ---- row log (make_bed --vo / -p summaries of the multi-GPU product path) ---------------------------------------------
+    def enable_row_log(self, n_feat=0, site_flags=None):
+        """Log every row the histogram counts (mc_rowlog_append): global row index, site slot, probability and, with
+        n_feat > 0, the first n_feat features.  site_flags (uint8 per site slot, host or device) restricts the log to the
+        flagged site slots; rows closed by another contig's line are always logged."""
+        if not (self.histogram and self.models is not None):
+            raise ValueError("the row log needs the histogram and the models")
+        self.log_nfeat = int(n_feat)
+        self.log_stride = int(self.L.mc_rowlog_stride(self.log_nfeat))
+        self.d_log_flags = None
+        if site_flags is not None:
+            self.d_log_flags = torch.as_tensor(np.ascontiguousarray(site_flags, dtype=np.uint8)).to(self.device)
+        self.log_cap = 0
+        # entries logged so far as the host knows them without a synchronisation of its own: the exact count from each
+        # chunk's status read (S_NLOG), a chunk's row capacity where no status is read
+        self.log_bound = 0
+        self.d_log = torch.empty(0, dtype=torch.uint8, device=self.device)
+        self.d_persist[P_N_LOG] = 0
+        self._log_room(1 << 16)
+
+    def _log_room(self, rows):
+        """Grow the log so that `rows` more entries fit after every entry that may have been logged so far."""
+        need = self.log_bound + int(rows)
+        if need <= self.log_cap:
+            return
+        cap = max(need, 2 * self.log_cap)
+        new = torch.empty(cap * self.log_stride, dtype=torch.uint8, device=self.device)
+        if self.log_cap:
+            new[:self.log_cap * self.log_stride].copy_(self.d_log)
+        self.d_log, self.log_cap = new, cap
+
+    def _log_rows(self, d_calls, d_nrows, row_cap, d_row_base, d_n_added, d_abort):
+        V = C.c_void_p
+        flags = V(self.d_log_flags.data_ptr()) if self.d_log_flags is not None else None
+        check(self.L.mc_rowlog_append(d_calls, d_nrows, row_cap, d_row_base, flags, self.ref.n_sites, self.log_nfeat,
+                                      V(self.d_log.data_ptr()), self.log_cap, self._persist_ptr(P_N_LOG), d_n_added, d_abort,
+                                      self._sptr()))
+        self.launches += 1
+
+    def row_log(self):
+        """(uint8 device tensor of the logged entries, their count) -- 8-byte D2H, synchronises."""
+        if self.d_log is None:
+            raise ValueError("the row log is not enabled")
+        n = int(self.d_persist[P_N_LOG].item())
+        if n > self.log_cap:
+            raise _lib.McallerCudaError("row log holds %d entries, capacity %d" % (n, self.log_cap))
+        return self.d_log[:n * self.log_stride], n
 
     def carry_state(self):
         """(open window carried out of the last chunk?, contig of the first kept line since the reset or -1) -- 16-byte D2H."""
@@ -173,6 +227,10 @@ class Engine(object):
                                     C.c_void_p(self.d_first.data_ptr()) if hist else None, self.ref.n_sites,
                                     self._persist_ptr(P_ROW_BASE), self._sptr()))
         self.launches += 1
+        if hist and self.d_log is not None:
+            self._log_room(1)
+            self._log_rows(C.c_void_p(self.d_carry_out.data_ptr()), None, 1, None, None, None)    # its index is in pad1/pad2
+            self.log_bound += 1
         if not fetch:
             return None
         return self.d_carry_out.cpu().numpy().view(CALL_DTYPE)
@@ -307,15 +365,26 @@ class Engine(object):
             check(L.mc_classify(V(calls.data_ptr()), self._status_ptr(S_NROWS), call_cap + 1, self.models.array, V(cls_ws.data_ptr()), st))
             self.launches += 2                       # index list of the call rows + the classifier
             if self.histogram:
+                if self.d_log is not None:
+                    # before mc_hist_accumulate, which advances the row base past this chunk
+                    self._log_room(call_cap + 1)
+                    self._log_rows(V(calls.data_ptr()), self._status_ptr(S_NROWS), call_cap + 1, self._persist_ptr(P_ROW_BASE),
+                                   self._status_ptr(S_NLOG), self._status_ptr(S_ABORT))
                 check(L.mc_hist_accumulate(V(calls.data_ptr()), self._status_ptr(S_NROWS), call_cap + 1, V(self.d_depth.data_ptr()),
                                            V(self.d_meth.data_ptr()), V(self.d_first.data_ptr()), self.ref.n_sites, self._persist_ptr(P_ROW_BASE),
                                            V(self.d_odd.data_ptr()), ODD_CAP, self._persist_ptr(P_N_ODD), self._status_ptr(S_ABORT), st))
                 self.launches += 2
         check(L.mc_count_calls(V(calls.data_ptr()), self._status_ptr(S_NROWS), call_cap + 1, self._status_ptr(S_STATS), st))
         self.launches += 1
+        log = self.d_log is not None and self.models is not None and self.histogram
         if not read_status:
+            if log:
+                self.log_bound += call_cap + 1
             return None
-        return self._read_status().copy()
+        cnt = self._read_status().copy()
+        if log:
+            self.log_bound += int(cnt[S_NLOG])            # 0 when the chunk overflowed and logged nothing
+        return cnt
 
     def launch_chunk(self, d_text, nbytes):
         """Queues every stage of a chunk WITHOUT reading its status: for back-to-back passes over inputs whose buffer needs are

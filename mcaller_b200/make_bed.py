@@ -61,9 +61,9 @@ def _fnv(parts):
     return h or 1
 
 
-def _pos_hash_set(pos_set):
-    """Open-addressing set of FNV-1a("chrom\\tpos\\tstrand") for the entries a row can match: the reference tests
-    (csome, pos, str(int(pos)+1), strand) in pos_set (:83-84), so an entry whose end column is not start + 1 never matches."""
+def _pos_keys(pos_set):
+    """(chrom, pos, strand) of the entries a row can match: the reference tests (csome, pos, str(int(pos)+1), strand) in
+    pos_set (:83-84), so an entry whose end column is not start + 1 never matches."""
     keys = set()
     for t in pos_set:
         if len(t) != 4:
@@ -74,7 +74,13 @@ def _pos_hash_set(pos_set):
                 continue
         except ValueError:
             continue
-        keys.add(_fnv([chrom.encode(), start.encode(), strand.encode()]))
+        keys.add((chrom, start, strand))
+    return keys
+
+
+def _pos_hash_set(pos_set):
+    """Open-addressing set of FNV-1a("chrom\\tpos\\tstrand") of _pos_keys(pos_set)."""
+    keys = set(_fnv([chrom.encode(), start.encode(), strand.encode()]) for chrom, start, strand in _pos_keys(pos_set))
     size = 64
     while size < 2 * len(keys) + 2:
         size *= 2
@@ -230,8 +236,6 @@ class _Aggregation(object):
 
     def column_tests(self):
         """values_dict[locus] of :115-127: [np.round(max t, 3), np.round(sum -log10 p, 3)] per locus."""
-        import warnings
-        from scipy import special
         torch, _lib = self.torch, self._lib
         n_loci = len(self.loci)
         if n_loci == 0:
@@ -258,22 +262,32 @@ class _Aggregation(object):
         self.vals = d_vals.cpu().numpy().reshape(self.n_rows, _lib.MC_MAXK + 1)     # parsed features, grouped row order
         if (ncol != ncols).any():
             raise ValueError("rows of %s do not all hold %d feature columns" % (self.path, ncols))
-        stats = d_stats.cpu().numpy().reshape(n_loci, ncols, 2)
-        n = (self.locus_off[1:].astype(np.int64) - self.locus_off[:-1].astype(np.int64)).astype(np.float64)[:, None]
-        out = []
-        with warnings.catch_warnings(), np.errstate(all="ignore"):
-            warnings.simplefilter("ignore")
-            # scipy.stats.ttest_1samp(x, 0): mean, _var = mean((x-mean)**2) * (n / (n-1)), t = mean / sqrt(var / n),
-            # p = 2 * stdtr(n-1, -|t|)
-            mean = stats[:, :, 0]
-            var = (stats[:, :, 1] / n) * (n / (n - 1.0))
-            t = mean / np.sqrt(var / n)
-            p = 2 * special.stdtr(n - 1.0, -np.abs(t))
-            for li in range(n_loci):
-                pvals = [(p[li, c], t[li, c]) for c in range(ncols)]
-                pval = (sum([-np.log10(x[0]) for x in pvals]), max([x[1] for x in pvals]))
-                out.append([np.round(x, 3) for x in [pval[1], pval[0]]])
-        return out
+        return ttest_finish(d_stats.cpu().numpy().reshape(n_loci, ncols, 2), self.locus_off)
+
+
+def ttest_finish(stats, locus_off):
+    """values_dict[locus] of :115-127 from the device statistics: stats[n_loci][ncols][2] = (np.mean(x), np.add.reduce((x -
+    mean)**2)) per locus and column, locus_off[n_loci + 1] the CSR of the rows -> [np.round(max t, 3), np.round(sum -log10 p,
+    3)] per locus (Student-t tail, -log10 and rounding as the reference's scipy / numpy calls)."""
+    import warnings
+    from scipy import special
+    n_loci, ncols = stats.shape[0], stats.shape[1]
+    locus_off = np.asarray(locus_off)
+    n = (locus_off[1:].astype(np.int64) - locus_off[:-1].astype(np.int64)).astype(np.float64)[:, None]
+    out = []
+    with warnings.catch_warnings(), np.errstate(all="ignore"):
+        warnings.simplefilter("ignore")
+        # scipy.stats.ttest_1samp(x, 0): mean, _var = mean((x-mean)**2) * (n / (n-1)), t = mean / sqrt(var / n),
+        # p = 2 * stdtr(n-1, -|t|)
+        mean = stats[:, :, 0]
+        var = (stats[:, :, 1] / n) * (n / (n - 1.0))
+        t = mean / np.sqrt(var / n)
+        p = 2 * special.stdtr(n - 1.0, -np.abs(t))
+        for li in range(n_loci):
+            pvals = [(p[li, c], t[li, c]) for c in range(ncols)]
+            pval = (sum([-np.log10(x[0]) for x in pvals]), max([x[1] for x in pvals]))
+            out.append([np.round(x, 3) for x in [pval[1], pval[0]]])
+    return out
 
 
 def count_loci(meth_fi):
@@ -359,21 +373,17 @@ def _write_loci(loci, aggfi, depth_thresh, mod_thresh, pos_list, control, verbos
     return count
 
 
-def loci_from_histogram(refindex, depth, meth, first, odd_rows=None):
-    """The per-site histogram of the fused pipeline (mc_hist_accumulate; all-reduced over the ranks of a multi-GPU run)
-    -> list of (chrom, pos, context, strand, depth, meth) in first-seen order, i.e. what make_bed.py:75-98 builds from
-    the `.diffs` rows.  A site slot IS the reference's key (chrom, pos, pos+1, context, strand): the context is a function of
-    contig, position and strand.  `odd_rows` (Engine.odd_rows(), gathered over ranks) are the rows whose column 1 names
-    another contig than their window's (reference quirk, extract_contexts.py:216): they form loci of their own."""
+def _locus_entries(refindex, depth, meth, first, odd_rows=None):
+    """Loci of the device histogram in first-seen order: (locus tuple, site slot or -1, global row indices of its odd rows)."""
     depth = np.asarray(depth).astype(np.int64)
     meth = np.asarray(meth).astype(np.int64)
     first = np.asarray(first).astype(np.uint64)
     used = np.flatnonzero(depth > 0)
-    entries = []                                  # (first-seen index, locus tuple)
+    entries = []                                  # (first-seen index, locus tuple, site slot, odd row indices)
     for s_ in used.tolist():
         ci, pos, rev = int(refindex.site_contig[s_]), int(refindex.site_pos[s_]), bool(refindex.site_rev[s_])
         entries.append((int(first[s_]), (refindex.names[ci], str(pos), refindex.context(ci, pos, rev), "-" if rev else "+",
-                                         int(depth[s_]), int(meth[s_]))))
+                                         int(depth[s_]), int(meth[s_])), s_, ()))
     if odd_rows is not None and len(odd_rows):
         extra = {}
         for c in odd_rows:
@@ -381,22 +391,156 @@ def loci_from_histogram(refindex, depth, meth, first, odd_rows=None):
             key = (refindex.names[int(c["chrom_contig"])], str(int(c["mpos"])), refindex.context(int(c["win_contig"]), int(c["mpos"]), rev),
                    "-" if rev else "+")
             idx = int(c["pad1"]) | (int(c["pad2"]) << 32)
-            e = extra.setdefault(key, [idx, 0, 0])
+            e = extra.setdefault(key, [idx, 0, 0, []])
             e[0] = min(e[0], idx)
             e[1] += 1
             e[2] += int(c["label"])
-        for key, (idx, d_, m_) in extra.items():
-            entries.append((idx, key + (d_, m_)))
+            e[3].append(idx)
+        for key, (idx, d_, m_, rows) in extra.items():
+            entries.append((idx, key + (d_, m_), -1, tuple(rows)))
     entries.sort(key=lambda t: t[0])
-    return [e[1] for e in entries]
+    return [e[1:] for e in entries]
+
+
+def loci_from_histogram(refindex, depth, meth, first, odd_rows=None):
+    """The per-site histogram of the fused pipeline (mc_hist_accumulate; all-reduced over the ranks of a multi-GPU run)
+    -> list of (chrom, pos, context, strand, depth, meth) in first-seen order, i.e. what make_bed.py:75-98 builds from
+    the `.diffs` rows.  A site slot IS the reference's key (chrom, pos, pos+1, context, strand): the context is a function of
+    contig, position and strand.  `odd_rows` (Engine.odd_rows(), gathered over ranks) are the rows whose column 1 names
+    another contig than their window's (reference quirk, extract_contexts.py:216): they form loci of their own."""
+    return [e[0] for e in _locus_entries(refindex, depth, meth, first, odd_rows)]
 
 
 def aggregate_from_histogram(refindex, depth, meth, first, aggfi, depth_thresh, mod_thresh, control=False, gff=False, ref=None,
                              odd_rows=None):
     """make_bed.py's default output (also --control / --gff / --ref) straight from the device histogram: no `.diffs` text is
-    parsed.  The modes that need per-read lists (-p, --vo) go through aggregate_by_pos on the `.diffs` file."""
+    parsed.  The modes that need per-read lists (-p, --vo) take the rows the ranks logged on the device as well:
+    aggregate_from_rows."""
     loci = loci_from_histogram(refindex, depth, meth, first, odd_rows)
     return _write_loci(loci, aggfi, depth_thresh, mod_thresh, None, control, False, gff, ref)
+
+
+def site_flags(refindex, pos_set):
+    """uint8 per site slot: 1 where the slot's (contig, str(pos), strand) -- the key a `.diffs` row of that site carries --
+    matches an entry of pos_set (make_pos_set) as make_bed.py:84 matches rows."""
+    flags = np.zeros(max(refindex.n_sites, 1), dtype=np.uint8)
+    names = {nm: i for i, nm in enumerate(refindex.names)}
+    g_site = refindex.contig_base[refindex.site_contig] + refindex.site_pos       # ascending within each strand
+    nf, ns = refindex.n_fwd, refindex.n_sites
+    for chrom, start, strand in _pos_keys(pos_set):
+        ci = names.get(chrom)
+        if ci is None or strand not in ("+", "-"):
+            continue
+        try:
+            pos = int(start)
+        except ValueError:
+            continue
+        if str(pos) != start or pos < 0 or pos >= int(refindex.contig_len[ci]):
+            continue
+        g = int(refindex.contig_base[ci]) + pos
+        lo, hi = (0, nf) if strand == "+" else (nf, ns)
+        j = lo + int(np.searchsorted(g_site[lo:hi], g))
+        if j < hi and int(g_site[j]) == g:
+            flags[j] = 1
+    return flags
+
+
+class _RowGroups(object):
+    """The per-locus row lists of the multi-GPU product path: the rows the ranks logged on the device (mc_rowlog_append),
+    gathered to this rank and grouped by locus on the device (mc_rowlog_group).  Offers what _write_loci takes from
+    _Aggregation -- prob_strings(li) -- and the t-test statistics of column_tests, with no `.diffs` text."""
+
+    def __init__(self, refindex, entries, d_log, n_log, n_feat, want_probs=True, want_vals=False):
+        import torch
+        from . import _lib
+        self.torch, self._lib, self.L = torch, _lib, _lib.lib()
+        dev = d_log.device
+        self.dev = dev
+        self.n_feat = int(n_feat)
+        n_loci = len(entries)
+        depth = np.zeros(n_loci + 1, dtype=np.uint32)
+        depth[:n_loci] = [e[0][4] for e in entries]
+        self.n_loci, self.n_rows = n_loci, int(depth.sum(dtype=np.int64))
+        locus_of_site = np.full(max(refindex.n_sites, 1), -1, dtype=np.int32)
+        odd_idx, odd_loc = [], []
+        for li, (_, site, rows) in enumerate(entries):
+            if site >= 0:
+                locus_of_site[site] = li
+            odd_idx += rows
+            odd_loc += [li] * len(rows)
+        o = np.argsort(np.array(odd_idx, dtype=np.uint64), kind="stable")
+        odd_rows = np.array(odd_idx, dtype=np.uint64)[o]
+        odd_locus = np.array(odd_loc, dtype=np.int32)[o]
+
+        def up(a):
+            return torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+
+        def p(t):
+            return C.c_void_p(t.data_ptr()) if t is not None else None
+        d_los, d_depth = up(locus_of_site), up(depth.view(np.int32))
+        d_odd_rows, d_odd_locus = up(odd_rows.view(np.int64) if len(odd_rows) else np.zeros(1, np.int64)), up(odd_locus if len(odd_locus) else np.zeros(1, np.int32))
+        d_off = torch.empty(n_loci + 1, dtype=torch.int32, device=dev)
+        self.d_prob = torch.empty(max(self.n_rows, 1), dtype=torch.float64, device=dev)
+        self.d_vals = self.d_ncol = None
+        if want_vals:
+            self.d_vals = torch.empty(max(self.n_rows, 1) * (_lib.MC_MAXK + 1), dtype=torch.float64, device=dev)
+            self.d_ncol = torch.empty(max(self.n_rows, 1), dtype=torch.int32, device=dev)
+        ws = torch.empty(int(self.L.mc_rowlog_group_workspace_bytes(self.n_rows, n_loci)), dtype=torch.uint8, device=dev)
+        d_cnt = torch.zeros(2, dtype=torch.int64, device=dev)
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(self.L.mc_rowlog_group(p(d_log), int(n_log), self.n_feat, p(d_los), refindex.n_sites, p(d_odd_rows), p(d_odd_locus),
+                                          len(odd_rows), p(d_depth), n_loci, self.n_rows, p(d_off), p(self.d_prob), p(self.d_vals),
+                                          p(self.d_ncol), p(ws), p(d_cnt), st))
+        self.d_off = d_off
+        cnt = d_cnt.cpu().numpy()
+        if cnt[1] or int(n_log) - int(cnt[0]) != self.n_rows:
+            raise _lib.McallerCudaError("the row log holds %d rows of the reported loci, the histogram counted %d"
+                                        % (int(n_log) - int(cnt[0]) - int(cnt[1]), self.n_rows))
+        self.locus_off = d_off.cpu().numpy().view(np.uint32)
+        self.text, self.offs = "", [0]
+        if want_probs and self.n_rows:
+            probs = self.d_prob[:self.n_rows].cpu().numpy()
+            buf = np.empty(32 * self.n_rows, dtype=np.uint8)
+            offs = np.empty(self.n_rows + 1, dtype=np.int64)
+            total = self.L.mc_format_probs(probs.ctypes.data_as(C.c_void_p), self.n_rows, 0, buf.ctypes.data_as(C.c_void_p), len(buf),
+                                           offs.ctypes.data_as(C.c_void_p))
+            if total < 0:
+                _lib.check(int(total))
+            self.text = buf[:total].tobytes().decode("ascii")
+            self.offs = offs.tolist()
+
+    def prob_strings(self, li):
+        """pos_dict_verbose[locus] (:96-97): the `.diffs` probability text of the locus's rows, file order."""
+        t, o = self.text, self.offs
+        return [t[o[j]:o[j + 1]] for j in range(int(self.locus_off[li]), int(self.locus_off[li + 1]))]
+
+    def column_tests(self):
+        """values_dict[locus] of :115-127 from the logged features (k columns: the trailing read quality is not logged, :91)."""
+        torch, _lib = self.torch, self._lib
+        if self.n_loci == 0:
+            return []
+        if self.d_vals is None or not (1 <= self.n_feat <= _lib.MC_MAXK):
+            raise ValueError("the row log holds no feature columns")
+        d_stats = torch.zeros(self.n_loci * self.n_feat * 2, dtype=torch.float64, device=self.dev)
+        _lib.check(self.L.mc_colstats(C.c_void_p(self.d_vals.data_ptr()), C.c_void_p(self.d_ncol.data_ptr()), C.c_void_p(self.d_off.data_ptr()),
+                                      self.n_loci, self.n_feat, C.c_void_p(d_stats.data_ptr()),
+                                      C.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)))
+        return ttest_finish(d_stats.cpu().numpy().reshape(self.n_loci, self.n_feat, 2), self.locus_off)
+
+
+def aggregate_from_rows(refindex, depth, meth, first, d_log, n_log, n_feat, aggfi, depth_thresh, mod_thresh, pos_list=None, control=False,
+                        verbose_results=False, gff=False, ref=None, odd_rows=None):
+    """make_bed.py --vo and -p (also with each other and with --gff / --control / --ref, combined as aggregate_by_pos combines
+    them) from the device histogram and the rows logged on the device (Engine.enable_row_log; gathered over the ranks of a
+    multi-GPU run, dist.gather_row_log): d_log holds n_log entries with n_feat features each (the k feature columns,
+    needed with pos_list).  No `.diffs` text is parsed."""
+    entries = _locus_entries(refindex, depth, meth, first, odd_rows)
+    if pos_list:
+        keys = _pos_keys(make_pos_set(pos_list))
+        entries = [e for e in entries if (e[0][0], e[0][1], e[0][3]) in keys]
+    groups = _RowGroups(refindex, entries, d_log, n_log, n_feat, want_probs=bool(verbose_results), want_vals=bool(pos_list))
+    tests = groups.column_tests() if pos_list else None
+    return _write_loci([e[0] for e in entries], aggfi, depth_thresh, mod_thresh, pos_list, control, verbose_results, gff, ref, groups, tests)
 
 
 def output_name(mCaller_file, positions=None, control=False, gff=False):

@@ -1,8 +1,12 @@
 """Multi-GPU run of the hot path on one eventalign file (SURVEY.md 8e): one process per GPU, rank r owns the reads whose
 first line lies in byte range r of N (the reference's `-t N` split, mCaller.py:63-68, snapped to read boundaries), writes
-its rows to `<prefix>.diffs.<k>.tmp<start>`, and the ranks exchange exactly two things over NCCL: the contig of each
-rank's first kept line (closes the previous rank's last window, extract_contexts.py:179) and the per-site histograms
-(make_bed.py:86-96), from which rank 0 writes the BED / GFF without ever parsing the `.diffs` text.
+its rows to `<prefix>.diffs.<k>.tmp<start>`, and the ranks exchange over NCCL the contig of each rank's first kept line
+(closes the previous rank's last window, extract_contexts.py:179) and the per-site histograms (make_bed.py:86-96), from
+which rank 0 writes the BED / GFF without ever parsing the `.diffs` text.  make_bed's per-read modes (`--bed_vo` = --vo,
+`--bed_positions FILE` = -p) also need each locus's rows: every rank then logs the rows its histogram counts on the device
+(probability, global row index, site slot and, with `--bed_positions`, the k features of the rows in that positions set),
+the logs are gathered to rank 0 (the third exchange, dist.gather_row_log), grouped by locus there on the device and
+handed to make_bed's BED writer.
 
     python -m mcaller_b200.cli mCaller -m GATC -r ref.fa -e x.eventalign.tsv -f x.fastq -d model.pkl --gpus 8 --bed
 
@@ -60,12 +64,18 @@ def run_rank(rank, world, port, a, backend=None):
         run = ec.RangeRun(a["tsv"], a["reference"], read2qual, a["k"], a["skip"], a["qual"], a["modelfile"], start, endline=end,
                           base=a["base"], motif=a["motif"], positions_list=a["positions"], histogram=True,
                           row_base=mdist.rank_row_base(rank))
+        bed_positions = a.get("bed_positions") if a.get("bed") else None
+        per_read = bool(a.get("bed") and (a.get("bed_vo") or bed_positions))
+        if per_read:                                  # make_bed --vo / -p: keep the rows of every locus (or of the listed ones)
+            flags = mb.site_flags(run.ref, mb.make_pos_set(bed_positions)) if bed_positions else None
+            run.eng.enable_row_log(a["k"] if bed_positions else 0, flags)
         import time
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         run.stream()
         torch.cuda.synchronize()
-        dt = time.perf_counter() - t0
+        t_streamed = time.perf_counter()
+        dt = t_streamed - t0
         print("rank %d: %.2f GB of eventalign text -> %d rows in %.2f s (%.1f GB/s, %.0f calls/s) on cuda:%d"
               % (rank, run.bytes_done / 1e9, run.sink.n_obs, dt, run.bytes_done / 1e9 / max(dt, 1e-9), run.sink.n_obs / max(dt, 1e-9), dev_index))
         eng = run.eng
@@ -73,13 +83,21 @@ def run_rank(rank, world, port, a, backend=None):
         run.consume_closed(mdist.close_and_reduce(eng, rank))
         odd = [None] * world
         dist.all_gather_object(odd, eng.odd_rows())
+        d_log, n_log = mdist.gather_row_log(eng, rank) if per_read else (None, 0)
         run.print_counters()
         if rank == 0 and a.get("bed"):
             odd_rows = np.concatenate(odd) if any(len(o) for o in odd) else None
-            out = mb.output_name(ec.diffs_name(a["tsv"], a["k"]), None, a["bed_control"], a["bed_gff"])
+            out = mb.output_name(ec.diffs_name(a["tsv"], a["k"]), bed_positions, a["bed_control"], a["bed_gff"])
             depth, meth, first = eng.histogram_host()
-            mb.aggregate_from_histogram(run.ref, depth, meth, first, out, a["bed_depth"], a["bed_thresh"], control=a["bed_control"],
-                                        gff=a["bed_gff"], ref=a["bed_ref"], odd_rows=odd_rows)
+            if per_read:
+                mb.aggregate_from_rows(run.ref, depth, meth, first, d_log, n_log, eng.log_nfeat, out, a["bed_depth"], a["bed_thresh"],
+                                       pos_list=bed_positions, control=a["bed_control"], verbose_results=a.get("bed_vo", False),
+                                       gff=a["bed_gff"], ref=a["bed_ref"], odd_rows=odd_rows)
+            else:
+                mb.aggregate_from_histogram(run.ref, depth, meth, first, out, a["bed_depth"], a["bed_thresh"], control=a["bed_control"],
+                                            gff=a["bed_gff"], ref=a["bed_ref"], odd_rows=odd_rows)
+            if per_read:
+                print("rank 0: %s written %.3f s after the end of streaming" % (out, time.perf_counter() - t_streamed))
         dist.barrier()
     finally:
         if own_group and dist.is_initialized():
